@@ -14,7 +14,9 @@ operator D [S, 5, n, n] with COLUMN-major n x n blocks, i.e. D[s, k, j, i] = D_r
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes
+import gc
 import math
 import os
 
@@ -37,6 +39,20 @@ def _ptr(t):
 
 def _stream():
     return torch.cuda.current_stream().cuda_stream
+
+
+@contextlib.contextmanager
+def _capture(graph):
+    """torch.cuda.graph with Python's cycle collector held off.  A dead hierarchy (MG <-> Level reference cycles) collected
+    mid-capture destroys its CUDA graphs and library context (cudaGraphExecDestroy, cudaFree), which invalidates the capture."""
+    enabled = gc.isenabled()
+    gc.disable()
+    try:
+        with torch.cuda.graph(graph):
+            yield
+    finally:
+        if enabled:
+            gc.enable()
 
 
 def D_to_reference_layout(D: torch.Tensor) -> torch.Tensor:
@@ -1019,7 +1035,7 @@ class CycleGraph:
                 lv.phi.copy_(ph); lv.r.copy_(r)
             self.graph = torch.cuda.CUDAGraph()
             n0 = mg.ctx.launches
-            with torch.cuda.graph(self.graph):
+            with _capture(self.graph):
                 self._body()
             self.nlaunch = mg.ctx.launches - n0
             for lv, ph, r in saved:      # capture does not execute, but keep the state explicit
@@ -1114,7 +1130,7 @@ class IterGraph:
                 t.copy_(c)
             self.graph = torch.cuda.CUDAGraph()
             n0 = sum(c.launches for c in mg._ctxs())
-            with torch.cuda.graph(self.graph):
+            with _capture(self.graph):
                 self.body(slot)
             self.nlaunch = sum(c.launches for c in mg._ctxs()) - n0
             for t, c in zip(self.state, saved):

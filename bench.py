@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run)
     python bench.py --impl reference ...                      (reference arm: the CPU path, see below)
+    python bench.py --gpus 1 ... --dump-outputs DIR           (also write the last timed solve's results as DIR/*.npy)
 
 A "step" is one full solve of D x = b (point source, x0 = 0) to |r|/|b| < 1e-10 on the workload lattice with
 the hierarchy already set up and all inputs resident in HBM.  `value` is the time to solution in ms
@@ -40,6 +41,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree (which may be read-only), bytecode caches included
 
 TOL = 1.0e-10
 METRIC = "wilson_mg_time_to_solution_1e-10"
@@ -282,6 +284,35 @@ def time_kernel(fn, reps, flush=None):
     return tot / reps
 
 
+DUMP_WINDOW = 256            # side of the block of sites around the point source stored in full
+DUMP_SAMPLE = 1 << 19        # sites of the fixed, seeded sample of the rest of the lattice
+DUMP_SEED = 20240601
+
+
+def dump_outputs(out_dir: str, x, info: dict, L: int):
+    """--dump-outputs: what the timed solve returned in its last step, as float64 .npy files, so that two builds can be
+    compared output for output.  The solution x [L*L, 2] complex128 (537 MB at 4096^2) is stored as (re, im) pairs on the
+    DUMP_WINDOW^2 sites around the point source (where it is large) and on a seeded sample of DUMP_SAMPLE sites (sorted site
+    indices, site = x + L*y, in x_sample_site.npy); the residual history and the recomputed true residual come from info."""
+    import numpy as np
+    import torch
+    w = min(L, DUMP_WINDOW)
+    rows = (L // 2 - w // 2 + np.arange(w)) % L
+    window = (rows[:, None] * L + rows[None, :]).reshape(-1)
+    sample = np.sort(np.random.default_rng(DUMP_SEED).choice(L * L, size=min(L * L, DUMP_SAMPLE), replace=False))
+
+    def pairs(sites):
+        v = x[torch.as_tensor(sites, device=x.device)].cpu().numpy()
+        return np.stack([v.real, v.imag], axis=-1).astype(np.float64)
+    out = {"x_window": pairs(window).reshape(w, w, 2, 2), "x_sample": pairs(sample), "x_sample_site": sample.astype(np.float64),
+           "resnorms": np.asarray(info["resnorms"], dtype=np.float64),
+           "true_resnorm": np.asarray([info["true_resnorm"]], dtype=np.float64)}
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def bind_to_gpu_numa_node(local: int):
     """Pin this process (and with it its first-touch / pinned host allocations) to the CPUs of the NUMA node the GPU hangs off:
     with 8 ranks copying their strips at the same time, host buffers on the wrong socket halve the copy bandwidth.
@@ -323,7 +354,13 @@ def main():
     ap.add_argument("--profile-step", action="store_true",
                     help="bracket ONE extra solve (+ one D-apply) with cudaProfilerStart/Stop for `ncu --profile-from-start off`; "
                          "numbers printed by such a run are not bench values")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed solve returned to DIR/<name>.npy (see dump_outputs; one GPU)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.gpus > 1 or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs is supported for the GPU solve on one GPU")
     if args.impl == "reference":
         run_reference_arm(args)
         return
@@ -435,6 +472,8 @@ def main():
         t = torch.tensor([ms], dtype=torch.float64, device=dev)
         torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
         ms = float(t.item())
+    if args.dump_outputs:           # now: x is LVL[0].phi, which the legs below overwrite
+        dump_outputs(args.dump_outputs, x, info, L)
 
     if args.profile_step:
         torch.cuda.synchronize()

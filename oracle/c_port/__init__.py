@@ -4,7 +4,9 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import stat
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -19,12 +21,25 @@ class _Level(C.Structure):
 
 
 def build() -> str:
+    """Path of an up-to-date libmgport.so: oracle/_ref/ of the tree, or a per-user temporary directory when the library there
+    is missing or stale and the tree is read-only."""
     src = os.path.join(_HERE, "mg_port.c")
-    if not os.path.exists(_SO) or os.path.getmtime(_SO) < os.path.getmtime(src):
-        os.makedirs(_OUT, exist_ok=True)
+    fresh = lambda so: os.path.exists(so) and os.path.getmtime(so) >= os.path.getmtime(src)
+    if fresh(_SO):
+        return _SO
+    out = _OUT if os.access(_OUT if os.path.isdir(_OUT) else os.path.dirname(_OUT), os.W_OK) else \
+        os.path.join(tempfile.gettempdir(), f"mg2d_c_port_{os.getuid()}")
+    if out != _OUT:
+        os.makedirs(out, mode=0o700, exist_ok=True)
+        st = os.lstat(out)          # a shared temporary directory: load nothing from a directory another account controls
+        if not stat.S_ISDIR(st.st_mode) or st.st_uid != os.getuid() or st.st_mode & 0o022:
+            raise RuntimeError(f"{out} is not a directory owned and writable only by this user")
+    so = os.path.join(out, "libmgport.so")
+    if not fresh(so):
+        os.makedirs(out, exist_ok=True)
         # baseline x86-64 ISA on purpose: the built library travels with the repo snapshot to a different host CPU
-        subprocess.check_call(["gcc", "-O3", "-fcx-limited-range", "-fopenmp", "-shared", "-fPIC", "-o", _SO, src, "-lm"])
-    return _SO
+        subprocess.check_call(["gcc", "-O3", "-fcx-limited-range", "-fopenmp", "-shared", "-fPIC", "-o", so, src, "-lm"])
+    return so
 
 
 def set_threads(n: int | None = None) -> int:

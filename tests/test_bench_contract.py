@@ -38,6 +38,34 @@ def test_reference_arm_other_ranks_are_silent(repo_root):
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_dump_outputs_files(repo_root, tmp_path, monkeypatch):
+    """--dump-outputs: float64 files only, the window centred on the point source, the same seeded sample on every call."""
+    import importlib.util
+    import torch
+    # loading bench.py runs its module-level settings: undo them when the test ends
+    monkeypatch.setattr(sys, "path", list(sys.path))
+    monkeypatch.setattr(sys, "dont_write_bytecode", sys.dont_write_bytecode)
+    spec = importlib.util.spec_from_file_location("bench_module", os.path.join(repo_root, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    L = 1024             # more sites than the sample takes
+    x = torch.complex(torch.arange(L * L * 2.0), -torch.arange(L * L * 2.0)).reshape(L * L, 2)
+    info = {"resnorms": [1.0, 1e-3, 1e-11], "true_resnorm": 2e-11}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), x, info, L)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["resnorms.npy", "true_resnorm.npy", "x_sample.npy", "x_sample_site.npy", "x_window.npy"]
+    for n in names:
+        a, b = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert a.dtype == np.float64 and np.array_equal(a, b), n
+    w = np.load(tmp_path / "a" / "x_window.npy")
+    c, h = L // 2, bench.DUMP_WINDOW // 2
+    assert w.shape == (2 * h, 2 * h, 2, 2) and tuple(w[h, h, 1]) == (2.0 * (c + c * L) + 1, -(2.0 * (c + c * L) + 1))
+    site = np.load(tmp_path / "a" / "x_sample_site.npy").astype(np.int64)
+    assert np.array_equal(np.load(tmp_path / "a" / "x_sample.npy")[:, 0, 0], 2.0 * site)
+    assert len(np.unique(site)) == len(site) == bench.DUMP_SAMPLE
+
+
 def test_refio_row_formats():
     L = 4
     phi = (np.arange(L * L * 2) + 1j * np.arange(L * L * 2)).reshape(L * L, 2)
