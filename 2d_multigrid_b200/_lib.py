@@ -21,6 +21,10 @@ _vp, _i, _d, _ll, _ull = C.c_void_p, C.c_int, C.c_double, C.c_longlong, C.c_ulon
 SIGNATURES = {
     "mg2d_wilson_apply": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _d, _i, _i, _i, _i, _vp, _vp],
     "mg2d_lvl0_matrix": [_vp, _vp, _vp, _d, _i, _i, _i, _i, _vp],
+    "mg2d_wilson_sw_apply": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _d, _i, _i, _i, _i, _vp, _vp],
+    "mg2d_wilson_sw_relax_rb": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _d, _i, _i, _i, _i, _i, _vp],
+    "mg2d_wilson_sw_relax_rb2": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _d, _i, _i, _i, _i, _vp, _vp],
+    "mg2d_clover_add": [_vp, _vp, _ll, _i, _vp],
     "mg2d_stencil_apply": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _ll, _ll, _vp, _vp],
     "mg2d_block_inverse": [_vp, _vp, _i, _ll, _i, _vp],
     "mg2d_relax_jacobi": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _ll, _ll, _vp],
@@ -74,6 +78,7 @@ SIGNATURES = {
     "mg2d_fill_uniform": [_vp, _ll, _ll, _ull, _ull, _d, _d, _i, _vp],
     "mg2d_gauge_metropolis": [_vp, _i, _d, _d, _i, _i, _ull, _ull, _vp],
     "mg2d_plaquette": [_vp, _i, _i, _vp, _vp],
+    "mg2d_clover_field": [_vp, _vp, _vp, _vp, _d, _i, _i, _i, _vp],
     "mg2d_phases_to_links": [_vp, _vp, _ll, _i, _vp],
     "mg2d_s2_relax": [_vp, _vp, _i, _d, _d, _i, _i, _vp],
     "mg2d_s2_project": [_vp, _vp, _vp, _i, _d, _d, _i, _vp],

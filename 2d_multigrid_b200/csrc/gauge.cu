@@ -8,6 +8,7 @@
 //                          such configurations, S6/gauge.h:44,88-110, beta in {6, 32}); mirrored draw-for-draw by
 //                          oracle gauge_quenched_phases_counter
 //   mg2d_plaquette         Gauge::f_plaquette, S6/gauge.h:50-63
+//   mg2d_clover_field      the real site field f(s) = (c_sw/8) sum_{P corner s} Im U_P of the clover self term (2+m) 1 + f s3
 //   mg2d_phases_to_links   U = polar(1, theta), S6/gauge.h:106
 #include "common.cuh"
 
@@ -82,6 +83,35 @@ plaquette_kernel(const cplx<T>* __restrict__ U, int L, double* __restrict__ part
     grid_reduce<2, 256>(red, partials, counter, out, blockIdx.x, gridDim.x);
 }
 
+// Im of the anticlockwise plaquette with base (x, y), y in [-1, Ly-1]: link rows -1 and Ly come from U_lo / U_hi
+template <typename T>
+__device__ __forceinline__ T im_plaquette(const cplx<T>* __restrict__ U, const cplx<T>* __restrict__ U_lo,
+                                          const cplx<T>* __restrict__ U_hi, int x, int y, int Lx, int Ly) {
+    using C = cplx<T>;
+    const int xp = (x + 1 == Lx) ? 0 : x + 1;
+    const C* r0 = (y < 0) ? U_lo : U + 2 * (size_t)y * Lx;                         // links of row y
+    const C* r1 = (y + 1 == Ly) ? U_hi : U + 2 * (size_t)(y + 1) * Lx;             // links of row y+1
+    const C ux = __ldg(r0 + 2 * x), uy = __ldg(r0 + 2 * x + 1), uy_x = __ldg(r0 + 2 * xp + 1), ux_y = __ldg(r1 + 2 * x);
+    // U_x(b) U_y(b+x) conj(U_x(b+y)) conj(U_y(b)), as in plaquette_kernel
+    const C a = cmul(ux, uy_x), b = cmul(ux_y, uy);
+    return cmulc(b, a).y;
+}
+
+// F[s] = (c_sw/8) (P(s) + P(s-x) + P(s-y) + P(s-x-y)), P(b) = Im U_P(b): the four plaquettes with a corner at s.  The same
+// operations in the same order at every site, so a strip gives its rows of the whole-lattice field bit for bit.
+template <typename T>
+__global__ void clover_field_kernel(T* __restrict__ F, const cplx<T>* __restrict__ U, const cplx<T>* __restrict__ U_lo,
+                                    const cplx<T>* __restrict__ U_hi, T c8, int Lx, int Ly) {
+    const long long S = (long long)Lx * Ly;
+    for (long long s = blockIdx.x * (long long)blockDim.x + threadIdx.x; s < S; s += (long long)gridDim.x * blockDim.x) {
+        const int y = (int)(s / Lx), x = (int)(s - (long long)y * Lx);
+        const int xm = (x == 0) ? Lx - 1 : x - 1;
+        const T p = im_plaquette<T>(U, U_lo, U_hi, x, y, Lx, Ly) + im_plaquette<T>(U, U_lo, U_hi, xm, y, Lx, Ly)
+                  + im_plaquette<T>(U, U_lo, U_hi, x, y - 1, Lx, Ly) + im_plaquette<T>(U, U_lo, U_hi, xm, y - 1, Lx, Ly);
+        F[s] = c8 * p;
+    }
+}
+
 template <typename T>
 __global__ void phases_to_links_kernel(cplx<T>* __restrict__ U, const double* __restrict__ theta, long long n) {
     for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
@@ -131,6 +161,19 @@ extern "C" int mg2d_plaquette(mg2d_ctx* ctx, const void* U, int L, int dtype, do
     else if (dtype == MG2D_C64) plaquette_kernel<float><<<grid, 256, 0, st>>>((const float2*)U, L, ctx->partials, ctx->counter, out);
     else return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_plaquette: bad dtype");
     return mg2d_check_launch(ctx, "mg2d_plaquette");
+}
+
+extern "C" int mg2d_clover_field(mg2d_ctx* ctx, void* F, const void* U, const void* U_lo, const void* U_hi, double csw, int Lx,
+                                 int Ly, int dtype, void* stream) {
+    if (!ctx) return MG2D_EINVAL;
+    if (!F || !U || !U_lo || !U_hi || Lx < 1 || Ly < 1) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_clover_field: bad argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int grid = grid_for(ctx, (long long)Lx * Ly);
+    const double c8 = csw / 8.0;
+    if (dtype == MG2D_C128) clover_field_kernel<double><<<grid, 256, 0, st>>>((double*)F, (const double2*)U, (const double2*)U_lo, (const double2*)U_hi, c8, Lx, Ly);
+    else if (dtype == MG2D_C64) clover_field_kernel<float><<<grid, 256, 0, st>>>((float*)F, (const float2*)U, (const float2*)U_lo, (const float2*)U_hi, (float)c8, Lx, Ly);
+    else return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_clover_field: bad dtype");
+    return mg2d_check_launch(ctx, "mg2d_clover_field");
 }
 
 extern "C" int mg2d_phases_to_links(mg2d_ctx* ctx, void* U, const double* theta, long long nelem, int dtype, void* stream) {

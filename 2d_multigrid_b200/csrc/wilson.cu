@@ -8,7 +8,11 @@
 //   1/2(1-s1)psi = 1/2 (a,-a),  a = psi0-psi1      1/2(1+s1)psi = 1/2 (b, b),  b = psi0+psi1
 //   1/2(1-s2)psi = 1/2 (c,-ic), c = psi0+i psi1    1/2(1+s2)psi = 1/2 (d, id), d = psi0-i psi1
 //
-// HBM roofline: algorithmic traffic 96 B/site in complex128 (psi in 32 + links 32 + out 32), +32 with b.
+// Clover (Sheikholeslami-Wohlert) variant, template flag SW: the self term becomes (2+m) 1 + f(s) s3 with the real site field
+// f of mg2d_clover_field (csrc/gauge.cu), i.e. (2+m+f) on component 0 and (2+m-f) on component 1.
+//
+// HBM roofline: algorithmic traffic 96 B/site in complex128 (psi in 32 + links 32 + out 32), +32 with b; SW adds f: 104 B/site
+// (c64: 48 -> 52).
 //
 // Kernel design (v1, "column march"): a CTA owns a strip of WX consecutive x and marches over RY rows in y.
 // Each thread keeps the three rows psi(x,y-1), psi(x,y), psi(x,y+1) and U_y(x,y-1) in registers, so every
@@ -23,15 +27,23 @@ namespace {
 constexpr int WX = 128;       // threads per CTA = x-extent of a CTA column strip
 constexpr int RY_MAX = 32;    // rows marched per work item (fewer on small lattices, to keep every SM busy)
 
-// MODE 0: out = D in ; MODE 1: out = b - D in.  DOTS: also reduce |out|^2, <out,in>, |b|^2.
-template <typename T, int MODE, bool DOTS>
-__global__ void __launch_bounds__(WX)
+// "<entry point>: <what>" (the Wilson and clover entry points share their argument checks)
+inline int mg2d_fail2(mg2d_ctx* ctx, const char* name, const char* what) {
+    snprintf(ctx->err, sizeof(ctx->err), "%s: %s", name, what);
+    return MG2D_EINVAL;
+}
+
+// MODE 0: out = D in ; MODE 1: out = b - D in.  DOTS: also reduce |out|^2, <out,in>, |b|^2.  SW: clover self term from F.
+// (the clover variants with DOTS ask for 5 CTAs per SM: left to its own heuristic ptxas spills the loop bound of the complex128
+// residual-norm variant; the Wilson instantiations keep the plain bound and their code)
+template <typename T, int MODE, bool DOTS, bool SW>
+__global__ void __launch_bounds__(WX, (SW && DOTS) ? 5 : 0)
 wilson_march_kernel(cplx<T>* __restrict__ out, const cplx<T>* __restrict__ in,
                     const cplx<T>* __restrict__ in_lo, const cplx<T>* __restrict__ in_hi,
                     const cplx<T>* __restrict__ U, const cplx<T>* __restrict__ U_lo,
                     const cplx<T>* __restrict__ b, T diag, int Lx, int Ly, int RY,
                     double* __restrict__ partials, unsigned int* __restrict__ counter,
-                    double* __restrict__ dots, XComm* xc) {
+                    double* __restrict__ dots, XComm* xc, const T* __restrict__ F) {
     using C = cplx<T>;
     const int nsx = (Lx + WX - 1) / WX;
     const int nsy = (Ly + RY - 1) / RY;
@@ -85,6 +97,11 @@ wilson_march_kernel(cplx<T>* __restrict__ out, const cplx<T>* __restrict__ in,
             C h1 = cadd(csub(B, A), cmul_i(csub(Dd, Cc)));
             o.c0.x = fma(diag, cur.c0.x, half * h0.x); o.c0.y = fma(diag, cur.c0.y, half * h0.y);
             o.c1.x = fma(diag, cur.c1.x, half * h1.x); o.c1.y = fma(diag, cur.c1.y, half * h1.y);
+            if (SW) {                                             // + f s3 psi(s)
+                const T f = __ldg(F + s);
+                o.c0.x = fma(f, cur.c0.x, o.c0.x); o.c0.y = fma(f, cur.c0.y, o.c0.y);
+                o.c1.x = fma(-f, cur.c1.x, o.c1.x); o.c1.y = fma(-f, cur.c1.y, o.c1.y);
+            }
             if (MODE == 1) {
                 Spinor<T> bb = load_spinor<T>(b, s);
                 if (DOTS && active) red[3] += (double)bb.c0.x * bb.c0.x + (double)bb.c0.y * bb.c0.y
@@ -111,12 +128,14 @@ wilson_march_kernel(cplx<T>* __restrict__ out, const cplx<T>* __restrict__ in,
 
 // red-black Gauss-Seidel half sweep, matrix-free: phi(s) = (r(s) - hop(s)) / (2+m) on the sites with
 // (x + y + yoff) % 2 == colour (f_relax's update, S6/level.h:116-121, with D0 = (2+m) 1).  One thread per
-// updated site; a warp covers 64 consecutive x.  Traffic per full sweep (c128): phi 32+32, r 32, links 2x32.
-template <typename T>
+// updated site; a warp covers 64 consecutive x.  Traffic per full sweep (c128): phi 32+32, r 32, links 2x32; SW: + f 8.
+// SW: D0 = diag(d+f, d-f), d = 2+m, inverted from one reciprocal 1/((d+f)(d-f)); a site with f == 0 uses inv_diag itself,
+// so c_sw = 0 reproduces the Wilson sweep bit for bit.
+template <typename T, bool SW>
 __global__ void __launch_bounds__(256)
 wilson_rb_kernel(cplx<T>* phi, const cplx<T>* lo, const cplx<T>* hi, const cplx<T>* __restrict__ U,
                  const cplx<T>* __restrict__ U_lo, const cplx<T>* __restrict__ r, T inv_diag, int Lx, int Ly,
-                 int colour, int yoff) {
+                 int colour, int yoff, const T* __restrict__ F, T diag) {
     using C = cplx<T>;
     const int Lh = Lx / 2;
     const long long S2 = (long long)Lh * Ly;
@@ -138,14 +157,19 @@ wilson_rb_kernel(cplx<T>* phi, const cplx<T>* lo, const cplx<T>* hi, const cplx<
         const C Dd = cmulc(uym, csub(qym.c0, cmul_i(qym.c1)));
         const C h0 = cadd(cadd(A, B), cadd(Cc, Dd));
         const C h1 = cadd(csub(B, A), cmul_i(csub(Dd, Cc)));
+        T i0 = inv_diag, i1 = inv_diag;
+        if (SW) {
+            const T f = __ldg(F + s);
+            if (f != (T)0) { const T q = (T)1 / ((diag + f) * (diag - f)); i0 = (diag - f) * q; i1 = (diag + f) * q; }
+        }
         Spinor<T> o;
         if (r) {
             const Spinor<T> rr = load_spinor<T>(r, s);
-            o.c0.x = (rr.c0.x - half * h0.x) * inv_diag; o.c0.y = (rr.c0.y - half * h0.y) * inv_diag;
-            o.c1.x = (rr.c1.x - half * h1.x) * inv_diag; o.c1.y = (rr.c1.y - half * h1.y) * inv_diag;
+            o.c0.x = (rr.c0.x - half * h0.x) * i0; o.c0.y = (rr.c0.y - half * h0.y) * i0;
+            o.c1.x = (rr.c1.x - half * h1.x) * i1; o.c1.y = (rr.c1.y - half * h1.y) * i1;
         } else {
-            o.c0.x = -half * h0.x * inv_diag; o.c0.y = -half * h0.y * inv_diag;
-            o.c1.x = -half * h1.x * inv_diag; o.c1.y = -half * h1.y * inv_diag;
+            o.c0.x = -half * h0.x * i0; o.c0.y = -half * h0.y * i0;
+            o.c1.x = -half * h1.x * i1; o.c1.y = -half * h1.y * i1;
         }
         store_spinor<T>(phi, s, o);
     }
@@ -187,10 +211,20 @@ __global__ void lvl0_matrix_kernel(cplx<T>* __restrict__ D, const cplx<T>* __res
     }
 }
 
+// clover term of the stored level-0 Wilson operator: D[s][0] += diag(F[s], -F[s])  (column-major: (0,0) at 0, (1,1) at 3)
+template <typename T>
+__global__ void clover_add_kernel(cplx<T>* __restrict__ D, const T* __restrict__ F, long long S) {
+    for (long long s = blockIdx.x * (long long)blockDim.x + threadIdx.x; s < S; s += (long long)gridDim.x * blockDim.x) {
+        const T f = F[s];
+        D[20 * s].x += f;
+        D[20 * s + 3].x -= f;
+    }
+}
+
 template <typename T>
 int launch_wilson(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo, const void* in_hi, const void* U,
-                  const void* U_lo, const void* b, double mass, int Lx, int Ly, int mode, double* dots,
-                  cudaStream_t st) {
+                  const void* U_lo, const void* F, const void* b, double mass, int Lx, int Ly, int mode, double* dots,
+                  cudaStream_t st, const char* name) {
     using C = cplx<T>;
     // rows per work item: as many as possible (each item re-reads 2 halo rows) while >= 6 CTAs per SM exist
     int RY = RY_MAX;
@@ -198,13 +232,52 @@ int launch_wilson(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo, c
     const int nwork = ((Lx + WX - 1) / WX) * ((Ly + RY - 1) / RY);
     int grid = nwork < MG2D_MAX_PARTIALS ? nwork : MG2D_MAX_PARTIALS;
     const T diag = (T)(2.0 + mass);
-#define WL(MODE, DOTS)                                                                                      \
-    wilson_march_kernel<T, MODE, DOTS><<<grid, WX, 0, st>>>((C*)out, (const C*)in, (const C*)in_lo,          \
-        (const C*)in_hi, (const C*)U, (const C*)U_lo, (const C*)b, diag, Lx, Ly, RY, ctx->partials, ctx->counter, dots, ctx->xreduce ? ctx->xcomm : nullptr)
-    if (mode == MG2D_MODE_APPLY) { if (dots) WL(0, true); else WL(0, false); }
-    else                         { if (dots) WL(1, true); else WL(1, false); }
+#define WL(MODE, DOTS, SW)                                                                                  \
+    wilson_march_kernel<T, MODE, DOTS, SW><<<grid, WX, 0, st>>>((C*)out, (const C*)in, (const C*)in_lo,      \
+        (const C*)in_hi, (const C*)U, (const C*)U_lo, (const C*)b, diag, Lx, Ly, RY, ctx->partials, ctx->counter, dots, \
+        ctx->xreduce ? ctx->xcomm : nullptr, (const T*)F)
+    if (F) {
+        if (mode == MG2D_MODE_APPLY) { if (dots) WL(0, true, true); else WL(0, false, true); }
+        else                         { if (dots) WL(1, true, true); else WL(1, false, true); }
+    } else {
+        if (mode == MG2D_MODE_APPLY) { if (dots) WL(0, true, false); else WL(0, false, false); }
+        else                         { if (dots) WL(1, true, false); else WL(1, false, false); }
+    }
 #undef WL
-    return mg2d_check_launch(ctx, "mg2d_wilson_apply");
+    return mg2d_check_launch(ctx, name);
+}
+
+int wilson_apply(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo, const void* in_hi, const void* U, const void* U_lo,
+                 const void* F, const void* b, double mass, int Lx, int Ly, int mode, int dtype, double* dots, void* stream,
+                 const char* name) {
+    if (!ctx) return MG2D_EINVAL;
+    if (!out || !in || !in_lo || !in_hi || !U || !U_lo || Lx < 2 || Ly < 1) return mg2d_fail2(ctx, name, "bad argument");
+    if (mode == MG2D_MODE_RESID && !b) return mg2d_fail2(ctx, name, "MODE_RESID needs b");
+    if (mode != MG2D_MODE_APPLY && mode != MG2D_MODE_RESID) return mg2d_fail2(ctx, name, "bad mode");
+    if (out == in) return mg2d_fail2(ctx, name, "out must not alias in");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype == MG2D_C128) return launch_wilson<double>(ctx, out, in, in_lo, in_hi, U, U_lo, F, b, mass, Lx, Ly, mode, dots, st, name);
+    if (dtype == MG2D_C64)  return launch_wilson<float>(ctx, out, in, in_lo, in_hi, U, U_lo, F, b, mass, Lx, Ly, mode, dots, st, name);
+    return mg2d_fail2(ctx, name, "bad dtype");
+}
+
+int wilson_relax_rb(mg2d_ctx* ctx, void* phi, const void* phi_lo, const void* phi_hi, const void* U, const void* U_lo,
+                    const void* F, const void* r, double mass, int Lx, int Ly, int colour, int yoff, int dtype, void* stream,
+                    const char* name) {
+    if (!ctx) return MG2D_EINVAL;
+    if (!phi || !phi_lo || !phi_hi || !U || !U_lo || Lx < 2 || (Lx & 1) || Ly < 1 || (colour != 0 && colour != 1))
+        return mg2d_fail2(ctx, name, "bad argument (Lx must be even)");
+    cudaStream_t st = (cudaStream_t)stream;
+    const long long S2 = (long long)(Lx / 2) * Ly;
+    long long nb = (S2 + 255) / 256; if (nb > (long long)ctx->num_sms * 32) nb = (long long)ctx->num_sms * 32;
+    const double inv = 1.0 / (2.0 + mass);
+#define RB(T, SW) wilson_rb_kernel<T, SW><<<(int)nb, 256, 0, st>>>((cplx<T>*)phi, (const cplx<T>*)phi_lo, (const cplx<T>*)phi_hi,  \
+        (const cplx<T>*)U, (const cplx<T>*)U_lo, (const cplx<T>*)r, (T)inv, Lx, Ly, colour, yoff, (const T*)F, (T)(2.0 + mass))
+    if (dtype == MG2D_C128) { if (F) RB(double, true); else RB(double, false); }
+    else if (dtype == MG2D_C64) { if (F) RB(float, true); else RB(float, false); }
+    else return mg2d_fail2(ctx, name, "bad dtype");
+#undef RB
+    return mg2d_check_launch(ctx, name);
 }
 
 }  // namespace
@@ -212,15 +285,14 @@ int launch_wilson(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo, c
 extern "C" int mg2d_wilson_apply(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo, const void* in_hi,
                                  const void* U, const void* U_lo, const void* b, double mass, int Lx, int Ly,
                                  int mode, int dtype, double* dots, void* stream) {
-    if (!ctx) return MG2D_EINVAL;
-    if (!out || !in || !in_lo || !in_hi || !U || !U_lo || Lx < 2 || Ly < 1) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_apply: bad argument");
-    if (mode == MG2D_MODE_RESID && !b) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_apply: MODE_RESID needs b");
-    if (mode != MG2D_MODE_APPLY && mode != MG2D_MODE_RESID) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_apply: bad mode");
-    if (out == in) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_apply: out must not alias in");
-    cudaStream_t st = (cudaStream_t)stream;
-    if (dtype == MG2D_C128) return launch_wilson<double>(ctx, out, in, in_lo, in_hi, U, U_lo, b, mass, Lx, Ly, mode, dots, st);
-    if (dtype == MG2D_C64)  return launch_wilson<float>(ctx, out, in, in_lo, in_hi, U, U_lo, b, mass, Lx, Ly, mode, dots, st);
-    return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_apply: bad dtype");
+    return wilson_apply(ctx, out, in, in_lo, in_hi, U, U_lo, nullptr, b, mass, Lx, Ly, mode, dtype, dots, stream, "mg2d_wilson_apply");
+}
+
+extern "C" int mg2d_wilson_sw_apply(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo, const void* in_hi,
+                                    const void* U, const void* U_lo, const void* F, const void* b, double mass, int Lx, int Ly,
+                                    int mode, int dtype, double* dots, void* stream) {
+    if (ctx && !F) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_sw_apply: F is NULL");
+    return wilson_apply(ctx, out, in, in_lo, in_hi, U, U_lo, F, b, mass, Lx, Ly, mode, dtype, dots, stream, "mg2d_wilson_sw_apply");
 }
 
 extern "C" int mg2d_lvl0_matrix(mg2d_ctx* ctx, void* D, const void* U, const void* U_lo, double mass, int stencil,
@@ -238,18 +310,26 @@ extern "C" int mg2d_lvl0_matrix(mg2d_ctx* ctx, void* D, const void* U, const voi
     return mg2d_check_launch(ctx, "mg2d_lvl0_matrix");
 }
 
+extern "C" int mg2d_clover_add(mg2d_ctx* ctx, void* D, const void* F, long long nsites, int dtype, void* stream) {
+    if (!ctx) return MG2D_EINVAL;
+    if (!D || !F || nsites < 1) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_clover_add: bad argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    long long grid = (nsites + 255) / 256; if (grid > (long long)ctx->num_sms * 8) grid = (long long)ctx->num_sms * 8;
+    if (dtype == MG2D_C128) clover_add_kernel<double><<<(int)grid, 256, 0, st>>>((double2*)D, (const double*)F, nsites);
+    else if (dtype == MG2D_C64) clover_add_kernel<float><<<(int)grid, 256, 0, st>>>((float2*)D, (const float*)F, nsites);
+    else return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_clover_add: bad dtype");
+    return mg2d_check_launch(ctx, "mg2d_clover_add");
+}
+
 extern "C" int mg2d_wilson_relax_rb(mg2d_ctx* ctx, void* phi, const void* phi_lo, const void* phi_hi, const void* U,
                                     const void* U_lo, const void* r, double mass, int Lx, int Ly, int colour, int yoff,
                                     int dtype, void* stream) {
-    if (!ctx) return MG2D_EINVAL;
-    if (!phi || !phi_lo || !phi_hi || !U || !U_lo || Lx < 2 || (Lx & 1) || Ly < 1 || (colour != 0 && colour != 1))
-        return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_relax_rb: bad argument (Lx must be even)");
-    cudaStream_t st = (cudaStream_t)stream;
-    const long long S2 = (long long)(Lx / 2) * Ly;
-    long long nb = (S2 + 255) / 256; if (nb > (long long)ctx->num_sms * 32) nb = (long long)ctx->num_sms * 32;
-    const double inv = 1.0 / (2.0 + mass);
-    if (dtype == MG2D_C128) wilson_rb_kernel<double><<<(int)nb, 256, 0, st>>>((double2*)phi, (const double2*)phi_lo, (const double2*)phi_hi, (const double2*)U, (const double2*)U_lo, (const double2*)r, inv, Lx, Ly, colour, yoff);
-    else if (dtype == MG2D_C64) wilson_rb_kernel<float><<<(int)nb, 256, 0, st>>>((float2*)phi, (const float2*)phi_lo, (const float2*)phi_hi, (const float2*)U, (const float2*)U_lo, (const float2*)r, (float)inv, Lx, Ly, colour, yoff);
-    else return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_relax_rb: bad dtype");
-    return mg2d_check_launch(ctx, "mg2d_wilson_relax_rb");
+    return wilson_relax_rb(ctx, phi, phi_lo, phi_hi, U, U_lo, nullptr, r, mass, Lx, Ly, colour, yoff, dtype, stream, "mg2d_wilson_relax_rb");
+}
+
+extern "C" int mg2d_wilson_sw_relax_rb(mg2d_ctx* ctx, void* phi, const void* phi_lo, const void* phi_hi, const void* U,
+                                       const void* U_lo, const void* F, const void* r, double mass, int Lx, int Ly, int colour,
+                                       int yoff, int dtype, void* stream) {
+    if (ctx && !F) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_sw_relax_rb: F is NULL");
+    return wilson_relax_rb(ctx, phi, phi_lo, phi_hi, U, U_lo, F, r, mass, Lx, Ly, colour, yoff, dtype, stream, "mg2d_wilson_sw_relax_rb");
 }

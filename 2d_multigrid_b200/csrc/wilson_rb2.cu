@@ -17,6 +17,10 @@
 // two-row halos `in_lo2` / `in_hi2`.  Old red values are never read.
 // Traffic per site and sweep (c128): phi 32 (read) + 32 (write) + links 32 + r 32 = 128 B, every byte of every
 // fetched line used (the half-sweep kernel: 160 B algorithmic, ~224 B moved).
+//
+// Clover variant (template flag SW): D0 = diag(d+f, d-f) with d = 2+m and the real site field f of mg2d_clover_field; every
+// update (halo rows and columns included) loads its site's f once and inverts D0 from one reciprocal 1/((d+f)(d-f)).  The red stage recomputes rows -1 and Ly, so strips pass f there as F_lo / F_hi.
+// Traffic: + f 8 B/site = 136 B (c64: 68 B).
 #include "common.cuh"
 #include "spinor.cuh"
 
@@ -34,6 +38,8 @@ struct Rb2Args {
     T inv_diag;
     int Lx, Ly, RY, yoff;
     HaloLinkDev link;      // strips: fused neighbour push / wait (mine == NULL: none)
+    const T* F; const T* F_lo; const T* F_hi;    // SW: clover field of the local rows, rows -1 and Ly
+    T diag;                                      // SW: 2+m
 };
 
 template <typename T>
@@ -52,11 +58,19 @@ __device__ __forceinline__ Spinor<T> rb2_phi(const Rb2Args<T>& a, int y, int x, 
     return load_spinor<T>(row, (size_t)x);
 }
 
+// clover field at (y, x), y in [-1, Ly]
+template <typename T>
+__device__ __forceinline__ T rb2_f(const Rb2Args<T>& a, int y, int x) {
+    const T* row = (y < 0) ? a.F_lo : (y >= a.Ly ? a.F_hi : a.F + (size_t)y * a.Lx);
+    return __ldg(row + x);
+}
+
 // phi(s) <- (r(s) - 1/2 hop(s)) / (2+m);  a_xp = (psi0 - psi1)(s+x), wb_xm = conj(U_x(s-x)) (psi0 + psi1)(s-x)
-template <typename T, bool HAS_R>
+// SW: component 0 divided by d+f, component 1 by d-f (f == 0: inv_diag itself, as in wilson_rb_kernel)
+template <typename T, bool HAS_R, bool SW>
 __device__ __forceinline__ Spinor<T> rb2_update(cplx<T> ux, cplx<T> a_xp, cplx<T> wb_xm, cplx<T> uy, const Spinor<T>& qyp,
                                                 cplx<T> uym, const Spinor<T>& qym, const cplx<T>* __restrict__ r_row, int x,
-                                                T inv_diag) {
+                                                T inv_diag, const Rb2Args<T>& a, int y) {
     using C = cplx<T>;
     const T half = (T)0.5;
     const C A = cmul(ux, a_xp);
@@ -65,14 +79,19 @@ __device__ __forceinline__ Spinor<T> rb2_update(cplx<T> ux, cplx<T> a_xp, cplx<T
     const C Dd = cmulc(uym, csub(qym.c0, cmul_i(qym.c1)));
     const C h0 = cadd(cadd(A, B), cadd(Cc, Dd));
     const C h1 = cadd(csub(B, A), cmul_i(csub(Dd, Cc)));
+    T i0 = inv_diag, i1 = inv_diag;
+    if (SW) {
+        const T f = rb2_f<T>(a, y, x), d = a.diag;
+        if (f != (T)0) { const T q = (T)1 / ((d + f) * (d - f)); i0 = (d - f) * q; i1 = (d + f) * q; }
+    }
     Spinor<T> o;
     if (HAS_R) {
         const Spinor<T> rr = load_spinor<T>(r_row, (size_t)x);
-        o.c0.x = (rr.c0.x - half * h0.x) * inv_diag; o.c0.y = (rr.c0.y - half * h0.y) * inv_diag;
-        o.c1.x = (rr.c1.x - half * h1.x) * inv_diag; o.c1.y = (rr.c1.y - half * h1.y) * inv_diag;
+        o.c0.x = (rr.c0.x - half * h0.x) * i0; o.c0.y = (rr.c0.y - half * h0.y) * i0;
+        o.c1.x = (rr.c1.x - half * h1.x) * i1; o.c1.y = (rr.c1.y - half * h1.y) * i1;
     } else {
-        o.c0.x = -half * h0.x * inv_diag; o.c0.y = -half * h0.y * inv_diag;
-        o.c1.x = -half * h1.x * inv_diag; o.c1.y = -half * h1.y * inv_diag;
+        o.c0.x = -half * h0.x * i0; o.c0.y = -half * h0.y * i0;
+        o.c1.x = -half * h1.x * i1; o.c1.y = -half * h1.y * i1;
     }
     return o;
 }
@@ -99,7 +118,7 @@ __device__ __forceinline__ void rb2_store(const Rb2Args<T>& a, int y, int x0, in
     }
 }
 
-template <typename T, bool HAS_R, bool LINKED>
+template <typename T, bool HAS_R, bool LINKED, bool SW>
 __global__ void __launch_bounds__(RB2_THREADS, 4)
 wilson_rb2_kernel(Rb2Args<T> a) {
     using C = cplx<T>;
@@ -179,13 +198,13 @@ wilson_rb2_kernel(Rb2Args<T> a) {
                 C a_xp = shfl_c(a_here, lane + 1);
                 if (lane == 31) { const Spinor<T> q = rb2_phi<T>(a, rho, xp_out, linked); a_xp = csub(q.c0, q.c1); }
                 const C wb = cmulc(u0_ux0, cadd(bk_0.c0, bk_0.c1));
-                rd_0 = rb2_update<T, HAS_R>(u0_ux1, a_xp, wb, u0_uy1, bk_p, um_uy1, bk_m, rrow, x1, a.inv_diag);
+                rd_0 = rb2_update<T, HAS_R, SW>(u0_ux1, a_xp, wb, u0_uy1, bk_p, um_uy1, bk_m, rrow, x1, a.inv_diag, a, rho);
                 if (do_black) {
                     // ---- stage B(rho-1): target c1 of row rho-1; red sources of that row sit in c0 (rd_m)
                     a_here = csub(rd_m.c0, rd_m.c1);
                     a_xp = shfl_c(a_here, lane + 1);
                     const C wbm = cmulc(um_ux0, cadd(rd_m.c0, rd_m.c1));
-                    const Spinor<T> nb = rb2_update<T, HAS_R>(um_ux1, a_xp, wbm, um_uy1, rd_0, umm_uy1, rd_mm, rrow_m, x1, a.inv_diag);
+                    const Spinor<T> nb = rb2_update<T, HAS_R, SW>(um_ux1, a_xp, wbm, um_uy1, rd_0, umm_uy1, rd_mm, rrow_m, x1, a.inv_diag, a, rho - 1);
                     rb2_store<T>(a, rho - 1, x0, x1, act0, act1, rd_m, nb, push_lo, push_hi);
                 }
             } else {
@@ -197,13 +216,13 @@ wilson_rb2_kernel(Rb2Args<T> a) {
                     wb_xm = cmulc(__ldg(urow + 2 * (size_t)xm_out), cadd(q.c0, q.c1));
                 }
                 const C ap = csub(bk_0.c0, bk_0.c1);
-                rd_0 = rb2_update<T, HAS_R>(u0_ux0, ap, wb_xm, u0_uy0, bk_p, um_uy0, bk_m, rrow, x0, a.inv_diag);
+                rd_0 = rb2_update<T, HAS_R, SW>(u0_ux0, ap, wb_xm, u0_uy0, bk_p, um_uy0, bk_m, rrow, x0, a.inv_diag, a, rho);
                 if (do_black) {
                     // ---- stage B(rho-1): target c0 of row rho-1; red sources of that row sit in c1 (rd_m)
                     wb_here = cmulc(um_ux1, cadd(rd_m.c0, rd_m.c1));
                     wb_xm = shfl_c(wb_here, lane - 1);
                     const C apm = csub(rd_m.c0, rd_m.c1);
-                    const Spinor<T> nb = rb2_update<T, HAS_R>(um_ux0, apm, wb_xm, um_uy0, rd_0, umm_uy0, rd_mm, rrow_m, x0, a.inv_diag);
+                    const Spinor<T> nb = rb2_update<T, HAS_R, SW>(um_ux0, apm, wb_xm, um_uy0, rd_0, umm_uy0, rd_mm, rrow_m, x0, a.inv_diag, a, rho - 1);
                     rb2_store<T>(a, rho - 1, x0, x1, act0, act1, nb, rd_m, push_lo, push_hi);
                 }
             }
@@ -233,8 +252,9 @@ wilson_rb2_kernel(Rb2Args<T> a) {
 
 template <typename T>
 int launch_rb2(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo2, const void* in_hi2, const void* U,
-               const void* U_lo2, const void* U_hi, const void* r, const void* r_lo, const void* r_hi, double mass,
-               int Lx, int Ly, int yoff, const mg2d_halo_link* link, cudaStream_t st) {
+               const void* U_lo2, const void* U_hi, const void* F, const void* F_lo, const void* F_hi, const void* r,
+               const void* r_lo, const void* r_hi, double mass, int Lx, int Ly, int yoff, const mg2d_halo_link* link,
+               cudaStream_t st, const char* name) {
     using C = cplx<T>;
     Rb2Args<T> a;
     memset(&a.link, 0, sizeof(a.link));
@@ -246,6 +266,8 @@ int launch_rb2(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo2, con
     a.U = (const C*)U; a.U_lo2 = (const C*)U_lo2; a.U_hi = (const C*)U_hi;
     a.r = (const C*)r; a.r_lo = (const C*)r_lo; a.r_hi = (const C*)r_hi;
     a.inv_diag = (T)(1.0 / (2.0 + mass));
+    a.F = (const T*)F; a.F_lo = (const T*)F_lo; a.F_hi = (const T*)F_hi;
+    a.diag = (T)(2.0 + mass);
     a.Lx = Lx; a.Ly = Ly; a.yoff = yoff;
     // rows per chunk: every chunk re-reads 3 rows of phi and 2 of the links, so as long as possible while the
     // machine stays full (>= 12 warps per SM)
@@ -258,14 +280,35 @@ int launch_rb2(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo2, con
     long long grid = (nitems + RB2_THREADS / 32 - 1) / (RB2_THREADS / 32);
     const long long cap = (long long)ctx->num_sms * 4;
     if (grid > cap) grid = cap;
-    if (link) {
-        if (r) wilson_rb2_kernel<T, true, true><<<(int)grid, RB2_THREADS, 0, st>>>(a);
-        else   wilson_rb2_kernel<T, false, true><<<(int)grid, RB2_THREADS, 0, st>>>(a);
-    } else {
-        if (r) wilson_rb2_kernel<T, true, false><<<(int)grid, RB2_THREADS, 0, st>>>(a);
-        else   wilson_rb2_kernel<T, false, false><<<(int)grid, RB2_THREADS, 0, st>>>(a);
+#define RB2(SW)                                                                                             \
+    if (link) {                                                                                             \
+        if (r) wilson_rb2_kernel<T, true, true, SW><<<(int)grid, RB2_THREADS, 0, st>>>(a);                  \
+        else   wilson_rb2_kernel<T, false, true, SW><<<(int)grid, RB2_THREADS, 0, st>>>(a);                 \
+    } else {                                                                                                \
+        if (r) wilson_rb2_kernel<T, true, false, SW><<<(int)grid, RB2_THREADS, 0, st>>>(a);                 \
+        else   wilson_rb2_kernel<T, false, false, SW><<<(int)grid, RB2_THREADS, 0, st>>>(a);                \
     }
-    return mg2d_check_launch(ctx, "mg2d_wilson_relax_rb2");
+    if (F) { RB2(true) } else { RB2(false) }
+#undef RB2
+    return mg2d_check_launch(ctx, name);
+}
+
+int wilson_relax_rb2(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo2, const void* in_hi2, const void* U,
+                     const void* U_lo2, const void* U_hi, const void* F, const void* F_lo, const void* F_hi, const void* r,
+                     const void* r_lo, const void* r_hi, double mass, int Lx, int Ly, int yoff, int dtype,
+                     const mg2d_halo_link* link, void* stream, const char* name) {
+    if (!ctx) return MG2D_EINVAL;
+    if (!out || !in || !in_lo2 || !in_hi2 || !U || !U_lo2 || !U_hi || Lx < 2 || (Lx & 1) || Ly < 2 || (r && (!r_lo || !r_hi)) ||
+        (link && (!link->slot_mine || !link->slot_prev || !link->slot_next || ((link->push_next_lo == nullptr) != (link->push_prev_hi == nullptr))))) {
+        snprintf(ctx->err, sizeof(ctx->err), "%s: bad argument (Lx even, Ly >= 2)", name);
+        return MG2D_EINVAL;
+    }
+    if (out == in) { snprintf(ctx->err, sizeof(ctx->err), "%s: out must not alias in", name); return MG2D_EINVAL; }
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype == MG2D_C128) return launch_rb2<double>(ctx, out, in, in_lo2, in_hi2, U, U_lo2, U_hi, F, F_lo, F_hi, r, r_lo, r_hi, mass, Lx, Ly, yoff, link, st, name);
+    if (dtype == MG2D_C64)  return launch_rb2<float>(ctx, out, in, in_lo2, in_hi2, U, U_lo2, U_hi, F, F_lo, F_hi, r, r_lo, r_hi, mass, Lx, Ly, yoff, link, st, name);
+    snprintf(ctx->err, sizeof(ctx->err), "%s: bad dtype", name);
+    return MG2D_EINVAL;
 }
 
 }  // namespace
@@ -274,13 +317,15 @@ extern "C" int mg2d_wilson_relax_rb2(mg2d_ctx* ctx, void* out, const void* in, c
                                      const void* U, const void* U_lo2, const void* U_hi, const void* r, const void* r_lo,
                                      const void* r_hi, double mass, int Lx, int Ly, int yoff, int dtype,
                                      const mg2d_halo_link* link, void* stream) {
-    if (!ctx) return MG2D_EINVAL;
-    if (!out || !in || !in_lo2 || !in_hi2 || !U || !U_lo2 || !U_hi || Lx < 2 || (Lx & 1) || Ly < 2 || (r && (!r_lo || !r_hi)) ||
-        (link && (!link->slot_mine || !link->slot_prev || !link->slot_next || ((link->push_next_lo == nullptr) != (link->push_prev_hi == nullptr)))))
-        return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_relax_rb2: bad argument (Lx even, Ly >= 2)");
-    if (out == in) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_relax_rb2: out must not alias in");
-    cudaStream_t st = (cudaStream_t)stream;
-    if (dtype == MG2D_C128) return launch_rb2<double>(ctx, out, in, in_lo2, in_hi2, U, U_lo2, U_hi, r, r_lo, r_hi, mass, Lx, Ly, yoff, link, st);
-    if (dtype == MG2D_C64)  return launch_rb2<float>(ctx, out, in, in_lo2, in_hi2, U, U_lo2, U_hi, r, r_lo, r_hi, mass, Lx, Ly, yoff, link, st);
-    return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_relax_rb2: bad dtype");
+    return wilson_relax_rb2(ctx, out, in, in_lo2, in_hi2, U, U_lo2, U_hi, nullptr, nullptr, nullptr, r, r_lo, r_hi, mass, Lx, Ly,
+                            yoff, dtype, link, stream, "mg2d_wilson_relax_rb2");
+}
+
+extern "C" int mg2d_wilson_sw_relax_rb2(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo2, const void* in_hi2,
+                                        const void* U, const void* U_lo2, const void* U_hi, const void* F, const void* F_lo,
+                                        const void* F_hi, const void* r, const void* r_lo, const void* r_hi, double mass, int Lx,
+                                        int Ly, int yoff, int dtype, const mg2d_halo_link* link, void* stream) {
+    if (ctx && (!F || !F_lo || !F_hi)) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_sw_relax_rb2: F, F_lo and F_hi are required");
+    return wilson_relax_rb2(ctx, out, in, in_lo2, in_hi2, U, U_lo2, U_hi, F, F_lo, F_hi, r, r_lo, r_hi, mass, Lx, Ly, yoff, dtype,
+                            link, stream, "mg2d_wilson_sw_relax_rb2");
 }

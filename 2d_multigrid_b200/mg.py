@@ -106,6 +106,8 @@ class Level:
         self.phi_null = None   # [S,nc,nf]
         self.phi_null_c = None # [S,nc,nf/2]: chirality-compacted copy used by restriction / prolongation (wilson)
         self.U = None          # level 0 only: links [S,2]
+        self.clover = None     # level 0 with csw != 0: real clover field f [S] (float64 / float32 with the field precision)
+        self._clover_halos = None
         self.matrix_free = False
         self._work = {}
 
@@ -182,10 +184,20 @@ class Level:
         assert self.lvl == 0
         self.U = U
         self.bind_link_halos(None)
+        self.clover = None
+        if p.csw != 0.0:
+            # clover self term (2+m) 1 + f sigma3: f of the local rows from the links (and their halo rows)
+            rdt = torch.float64 if mg.dcode == _lib.C128 else torch.float32
+            self.clover = torch.empty(self.S, dtype=rdt, device=mg.device)
+            mg.ctx.call("mg2d_clover_field", _ptr(self.clover), _ptr(U), self.U_lo_ptr, self.U_hi_ptr, float(p.csw), self.L,
+                        self.Ly, mg.dcode, _stream())
+            self.bind_clover_halos(None)
         if store:
             self.D = torch.empty((self.S, 5, self.n, self.n), dtype=mg.tdtype, device=mg.device)
             mg.ctx.call("mg2d_lvl0_matrix", _ptr(self.D), _ptr(U), self.U_lo_ptr, float(p.mass),
                         0 if p.stencil == "wilson" else 1, self.L, self.Ly, mg.dcode, _stream())
+            if self.clover is not None:
+                mg.ctx.call("mg2d_clover_add", _ptr(self.D), _ptr(self.clover), self.S, mg.dcode, _stream())
             self.D0inv = None
             self.M = None
         self.matrix_free = not store
@@ -207,6 +219,20 @@ class Level:
             self.U_lo2_ptr, self.U_hi_ptr = U.data_ptr() + (self.Ly - 2) * row, U.data_ptr()
         self.U_lo_ptr = self.U_lo2_ptr + row          # row -1
 
+    def bind_clover_halos(self, halos):
+        """Rows -1 and Ly of the clover field (the two-colour sweep recomputes red sites there).  Exchanged once per gauge
+        field (halos None) or taken from `halos` = (lo, hi) tensors (precision copies); on one GPU the periodic wrap rows."""
+        F = self.clover
+        if self.distributed:
+            if halos is None:
+                lo, hi = self.mg.comm.exchange_rows(F, self.L, self.Ly, 1, 1, key=("clover",), as_tensor=True, depth=1)
+                halos = (lo.clone(), hi.clone())
+            self._clover_halos = halos
+            self.clover_lo_ptr, self.clover_hi_ptr = halos[0].data_ptr(), halos[1].data_ptr()
+        else:
+            self._clover_halos = None
+            self.clover_lo_ptr, self.clover_hi_ptr = F.data_ptr() + (self.Ly - 1) * self.L * F.element_size(), F.data_ptr()
+
     def _stencil(self, out, vin, b, mode, dots, nvec=1):
         mg = self.mg
         _lib.TRACE_TAG = self.lvl
@@ -219,8 +245,12 @@ class Level:
                                   None if dots is None else dots[4 * v:], 1)
                 return
             lo, hi = self._halo(vin)
-            mg.ctx.call("mg2d_wilson_apply", _ptr(out), _ptr(vin), lo, hi, _ptr(self.U), self.U_lo_ptr, _ptr(b),
-                        float(mg.p.mass), self.L, self.Ly, mode, mg.dcode, _ptr(dots), _stream())
+            if self.clover is None:
+                mg.ctx.call("mg2d_wilson_apply", _ptr(out), _ptr(vin), lo, hi, _ptr(self.U), self.U_lo_ptr, _ptr(b),
+                            float(mg.p.mass), self.L, self.Ly, mode, mg.dcode, _ptr(dots), _stream())
+            else:
+                mg.ctx.call("mg2d_wilson_sw_apply", _ptr(out), _ptr(vin), lo, hi, _ptr(self.U), self.U_lo_ptr, _ptr(self.clover),
+                            _ptr(b), float(mg.p.mass), self.L, self.Ly, mode, mg.dcode, _ptr(dots), _stream())
         else:
             vs = self.S * self.n
             lo, hi = self._halo(vin, nvec)
@@ -375,9 +405,14 @@ class Level:
                         link = ctypes.byref(lk)
                     else:
                         lo2, hi2 = self._halo(cur, depth=2)
-                    mg.ctx.call("mg2d_wilson_relax_rb2", _ptr(nxt), _ptr(cur), lo2, hi2, _ptr(self.U), self.U_lo2_ptr,
-                                self.U_hi_ptr, _ptr(rv), r_lo, r_hi, float(mg.p.mass), self.L, self.Ly, self.y0 & 1,
-                                mg.dcode, link, _stream())
+                    if self.clover is None:
+                        mg.ctx.call("mg2d_wilson_relax_rb2", _ptr(nxt), _ptr(cur), lo2, hi2, _ptr(self.U), self.U_lo2_ptr,
+                                    self.U_hi_ptr, _ptr(rv), r_lo, r_hi, float(mg.p.mass), self.L, self.Ly, self.y0 & 1,
+                                    mg.dcode, link, _stream())
+                    else:
+                        mg.ctx.call("mg2d_wilson_sw_relax_rb2", _ptr(nxt), _ptr(cur), lo2, hi2, _ptr(self.U), self.U_lo2_ptr,
+                                    self.U_hi_ptr, _ptr(self.clover), self.clover_lo_ptr, self.clover_hi_ptr, _ptr(rv), r_lo,
+                                    r_hi, float(mg.p.mass), self.L, self.Ly, self.y0 & 1, mg.dcode, link, _stream())
                     cur, nxt = nxt, cur
                 if num_iter & 1:
                     mg.ctx.call("mg2d_copy", _ptr(nxt), _ptr(cur), vs, mg.dcode, _stream())
@@ -397,8 +432,13 @@ class Level:
                             ph = phi if nvec == 1 else phi[v]
                             rv = None if r is None else (r if nvec == 1 else r[v])
                             lo, hi = self._halo(ph)
-                            mg.ctx.call("mg2d_wilson_relax_rb", _ptr(ph), lo, hi, _ptr(self.U), self.U_lo_ptr, _ptr(rv),
-                                        float(mg.p.mass), self.L, self.Ly, colour, self.y0 & 1, mg.dcode, _stream())
+                            if self.clover is None:
+                                mg.ctx.call("mg2d_wilson_relax_rb", _ptr(ph), lo, hi, _ptr(self.U), self.U_lo_ptr, _ptr(rv),
+                                            float(mg.p.mass), self.L, self.Ly, colour, self.y0 & 1, mg.dcode, _stream())
+                            else:
+                                mg.ctx.call("mg2d_wilson_sw_relax_rb", _ptr(ph), lo, hi, _ptr(self.U), self.U_lo_ptr,
+                                            _ptr(self.clover), _ptr(rv), float(mg.p.mass), self.L, self.Ly, colour, self.y0 & 1,
+                                            mg.dcode, _stream())
                     elif self.lr_rank and mg.premul and mg.lowrank and self._ensure_F():
                         # first coarse level: rank-`block` factors of the pre-multiplied hopping blocks (half the bytes);
                         # batches of 4 vectors share one stream of the factors (near-null generation)
@@ -629,7 +669,7 @@ class MG:
         allocator immediately (hierarchies are tens of GB)."""
         for lv in self.LVL + [nt for row in self.NTL for nt in row]:
             lv.__dict__.update(phi=None, r=None, D=None, D0inv=None, M=None, F=None, _lr_AB=None, Dh=None, D0inv_h=None, phi_null=None, phi_null_c=None,
-                               U=None, _U_halos=None, _work={}, mg=None)
+                               U=None, _U_halos=None, clover=None, _clover_halos=None, _work={}, mg=None)
         for v in list(self.info.values()):
             if isinstance(v, MG):
                 v.close()
@@ -682,7 +722,7 @@ class MG:
 
 
 def make_single_precision(mg: "MG") -> "MG":
-    """complex64 shadow of a set-up hierarchy (links, stored operators, projectors), used as the preconditioner
+    """complex64 shadow of a set-up hierarchy (links, clover field, stored operators, projectors), used as the preconditioner
     of the fp64 outer GCR: every V-cycle kernel then moves half the bytes.  The outer residual, the GCR vectors
     and the convergence test stay in complex128, so the 1e-10 TRUE residual is unaffected."""
     import dataclasses
@@ -709,6 +749,9 @@ def make_single_precision(mg: "MG") -> "MG":
         if lv.U is not None:
             l32.U = lv.U.to(c64)
             l32.bind_link_halos(None if lv._U_halos is None else tuple(h.to(c64) for h in lv._U_halos))
+        if lv.clover is not None:
+            l32.clover = lv.clover.to(torch.float32)
+            l32.bind_clover_halos(None if lv._clover_halos is None else tuple(h.to(torch.float32) for h in lv._clover_halos))
     return m32
 
 

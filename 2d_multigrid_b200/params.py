@@ -45,6 +45,8 @@ class MGParams:
     chiral_transfer: bool = True     # wilson: restriction / prolongation on the chirality-compacted projector
     matrix_free: bool | None = None  # level-0 Wilson operator applied from the links (no D0 stored).
                                      # default: True for smoother 'mr', False for 'gs'/'jacobi' (they need D0)
+    csw: float = 0.0                 # clover (Sheikholeslami-Wohlert) coefficient of the level-0 Wilson operator: self block
+                                     # (2+m) 1 + f(s) sigma3, f(s) = (csw/8) sum of Im U_P over the 4 plaquettes at s; 1 = tree level
     size: list = field(default_factory=list)
     n_dof: list = field(default_factory=list)
 
@@ -95,6 +97,12 @@ class MGParams:
             self.matrix_free = self.stencil == "wilson" and self.smoother in ("mr", "rbgs")
         if self.matrix_free and (self.stencil != "wilson" or self.smoother not in ("mr", "rbgs")):
             raise ValueError("matrix_free needs stencil='wilson' and smoother 'mr' or 'rbgs'")
+        self.csw = float(self.csw)
+        if self.csw != 0.0 and self.stencil != "wilson":
+            raise ValueError("the clover term (csw != 0) exists for stencil='wilson' only")
+        if self.csw != 0.0 and not 2.0 + self.mass - abs(self.csw) / 2.0 > 0.0:
+            # |f| <= |csw|/2, so this bound keeps every clover self block diag(2+m+f, 2+m-f) invertible
+            raise ValueError(f"clover self blocks may be singular: need 2 + mass - |csw|/2 > 0 (mass {self.mass}, csw {self.csw})")
 
     @property
     def diag(self) -> float:

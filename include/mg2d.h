@@ -64,6 +64,24 @@ int mg2d_wilson_apply(mg2d_ctx*, void* out, const void* in, const void* in_lo, c
  * stencil 0 = wilson (n=2), 1 = gauged laplace (n=1). */
 int mg2d_lvl0_matrix(mg2d_ctx*, void* D, const void* U, const void* U_lo, double mass, int stencil,
                      int Lx, int Ly, int dtype, void* stream);
+/* Wilson-clover (Sheikholeslami-Wohlert) level 0: the self block becomes (2+m) 1 + f(s) s3 with the real field
+ * f = F[s] of mg2d_clover_field (double for MG2D_C128, float for MG2D_C64; F_lo / F_hi = its rows -1 / Ly).
+ *   mg2d_wilson_sw_apply       mg2d_wilson_apply with the clover self term (APPLY, RESID, fused dots)
+ *   mg2d_wilson_sw_relax_rb    mg2d_wilson_relax_rb with D0 = diag(2+m+f, 2+m-f)
+ *   mg2d_wilson_sw_relax_rb2   mg2d_wilson_relax_rb2 with D0 = diag(2+m+f, 2+m-f); the red stage recomputes rows -1
+ *                              and Ly, hence F_lo / F_hi
+ *   mg2d_clover_add            stored operator: D[s][0] += diag(F[s], -F[s]) on nsites sites (stencil 0 blocks) */
+int mg2d_wilson_sw_apply(mg2d_ctx*, void* out, const void* in, const void* in_lo, const void* in_hi,
+                         const void* U, const void* U_lo, const void* F, const void* b, double mass, int Lx, int Ly,
+                         int mode, int dtype, double* dots, void* stream);
+int mg2d_wilson_sw_relax_rb(mg2d_ctx*, void* phi, const void* phi_lo, const void* phi_hi, const void* U,
+                            const void* U_lo, const void* F, const void* r, double mass, int Lx, int Ly, int colour,
+                            int yoff, int dtype, void* stream);
+int mg2d_wilson_sw_relax_rb2(mg2d_ctx*, void* out, const void* in, const void* in_lo2, const void* in_hi2,
+                             const void* U, const void* U_lo2, const void* U_hi, const void* F, const void* F_lo,
+                             const void* F_hi, const void* r, const void* r_lo, const void* r_hi, double mass, int Lx,
+                             int Ly, int yoff, int dtype, const struct mg2d_halo_link* link, void* stream);
+int mg2d_clover_add(mg2d_ctx*, void* D, const void* F, long long nsites, int dtype, void* stream);
 
 /* ---- generic 5-point block stencil (all coarse levels; level 0 in reference-compat mode) -------------- */
 /* Level::f_apply_D / f_residue, n in {1,2,4,8,16,32}; nvec vectors `vstride` elements apart. */
@@ -297,6 +315,11 @@ int mg2d_gauge_metropolis(mg2d_ctx*, double* theta, int L, double beta, double d
                           unsigned long long seed, unsigned long long tag, void* stream);
 /* Gauge::f_plaquette (S6/gauge.h:50-63): out[0..1] = sum_s U_x(s) U_y(s+x) conj(U_x(s+y)) conj(U_y(s)) (re, im). */
 int mg2d_plaquette(mg2d_ctx*, const void* U, int L, int dtype, double* out, void* stream);
+/* clover field of rows [0, Ly) of an Lx-wide strip: F[s] = (csw/8) sum over the four plaquettes P with a corner at s of
+ * Im U_P, U_P = U_x(b) U_y(b+x) conj(U_x(b+y)) conj(U_y(b)) (the orientation of mg2d_plaquette).  U_lo / U_hi = link rows
+ * -1 / Ly (on one GPU the periodic wrap rows of U).  A strip gets its rows of the whole-lattice field bit for bit. */
+int mg2d_clover_field(mg2d_ctx*, void* F, const void* U, const void* U_lo, const void* U_hi, double csw, int Lx, int Ly,
+                      int dtype, void* stream);
 /* U[e] = polar(1, theta[e]) (S6/gauge.h:106) */
 int mg2d_phases_to_links(mg2d_ctx*, void* U, const double* theta, long long nelem, int dtype, void* stream);
 
