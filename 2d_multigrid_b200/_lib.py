@@ -60,7 +60,7 @@ SIGNATURES = {
     "mg2d_restrict_chiral": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp],
     "mg2d_prolong_chiral": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp],
     "mg2d_pack_null": [_vp, _vp, _i, _ll, _i, _i, _ll, _i, _i, _vp],
-    "mg2d_norm_nn": [_vp, _i, _i, _i, _i, _i, _i, _i, _vp],
+    "mg2d_norm_nn": [_vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp],
     "mg2d_ortho": [_vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp],
     "mg2d_check_ortho": [_vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp],
     "mg2d_coarse_matrix": [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp],

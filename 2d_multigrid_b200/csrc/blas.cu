@@ -222,13 +222,11 @@ extern "C" int mg2d_create(mg2d_ctx** out, int device) {
     if (prop.major != 10) return MG2D_EUNSUPPORTED;   // sm_100a only: no fallback path exists
     mg2d_ctx* c = new mg2d_ctx();
     c->device = device; c->launches = 0; c->num_sms = prop.multiProcessorCount; c->err[0] = 0;
-    c->partials = nullptr; c->counter = nullptr; c->status = nullptr; c->xcomm = nullptr; c->xreduce = 0;
+    c->partials = nullptr; c->counter = nullptr; c->xcomm = nullptr; c->xreduce = 0;
     if (cudaMalloc(&c->partials, sizeof(double) * MG2D_MAX_PARTIALS * 4 * 64) != cudaSuccess ||
         cudaMalloc(&c->counter, sizeof(unsigned int) * 256) != cudaSuccess ||
-        cudaMalloc(&c->status, sizeof(int) * 16) != cudaSuccess ||
-        cudaMemset(c->counter, 0, sizeof(unsigned int) * 256) != cudaSuccess ||
-        cudaMemset(c->status, 0, sizeof(int) * 16) != cudaSuccess) {
-        cudaFree(c->partials); cudaFree(c->counter); cudaFree(c->status); delete c;
+        cudaMemset(c->counter, 0, sizeof(unsigned int) * 256) != cudaSuccess) {
+        cudaFree(c->partials); cudaFree(c->counter); delete c;
         return MG2D_ECUDA;
     }
     *out = c;
@@ -238,7 +236,7 @@ extern "C" int mg2d_create(mg2d_ctx** out, int device) {
 extern "C" int mg2d_destroy(mg2d_ctx* c) {
     if (!c) return MG2D_EINVAL;
     cudaSetDevice(c->device);
-    cudaFree(c->partials); cudaFree(c->counter); cudaFree(c->status);
+    cudaFree(c->partials); cudaFree(c->counter);
     delete c;
     return MG2D_OK;
 }

@@ -59,7 +59,6 @@ struct mg2d_ctx {
     int launches;
     double* partials;        // [MG2D_MAX_PARTIALS][MG2D_MAX_RED]
     unsigned int* counter;   // last-block-done tickets, one per reduction "channel"
-    int* status;
     int num_sms;
     XComm* xcomm;            // multi-GPU: descriptor for reductions fused into the kernels (NULL on one GPU)
     int xreduce;             // 1: reductions of the following calls are summed over all ranks inside the kernel

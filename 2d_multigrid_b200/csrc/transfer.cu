@@ -580,8 +580,9 @@ static int launch_rows(mg2d_ctx* ctx, void* P, int nf, int nc, int Lxf, int Lyf,
     return mg2d_check_launch(ctx, name);
 }
 
-extern "C" int mg2d_norm_nn(mg2d_ctx* ctx, void* P, int nf, int nc, int Lxf, int Lyf, int block, int quad, int dtype, void* stream) {
-    return launch_rows<0>(ctx, P, nf, nc, Lxf, Lyf, block, quad, dtype, ctx ? ctx->status : nullptr, nullptr, stream, "mg2d_norm_nn");
+extern "C" int mg2d_norm_nn(mg2d_ctx* ctx, void* P, int nf, int nc, int Lxf, int Lyf, int block, int quad, int dtype,
+                            int* status, void* stream) {
+    return launch_rows<0>(ctx, P, nf, nc, Lxf, Lyf, block, quad, dtype, status, nullptr, stream, "mg2d_norm_nn");
 }
 extern "C" int mg2d_ortho(mg2d_ctx* ctx, void* P, int nf, int nc, int Lxf, int Lyf, int block, int quad, int dtype,
                           int* status, void* stream) {

@@ -244,8 +244,10 @@ int mg2d_prolong_chiral(mg2d_ctx*, void* vf, void* vc, const void* Pc, int nf, i
 int mg2d_pack_null(mg2d_ctx*, void* P, const void* V, int nvec, long long vstride, int nf, int nc,
                    long long nsites, int wilson, int dtype, void* stream);
 /* Near_null::f_norm_nn (S6/near_null.h:24-48, f_block_norm S6/modules_indiv.h:94-135): every row of P
- * normalised per aggregate. */
-int mg2d_norm_nn(mg2d_ctx*, void* P, int nf, int nc, int Lxf, int Lyf, int block, int quad, int dtype, void* stream);
+ * normalised per aggregate.  `status` (device int, may be NULL) gets bit 1 when a block norm is NaN or below 1e-40
+ * (the reference exits there, S6/modules_indiv.h:119-126). */
+int mg2d_norm_nn(mg2d_ctx*, void* P, int nf, int nc, int Lxf, int Lyf, int block, int quad, int dtype,
+                 int* status, void* stream);
 /* Near_null::f_ortho (S6/near_null.h:97-173): per-aggregate modified Gram-Schmidt, t -= (dot/|u|) u, then
  * block-normalise.  `status` (device int, may be NULL) is set non-zero on NaN / tiny norms (:149-159). */
 int mg2d_ortho(mg2d_ctx*, void* P, int nf, int nc, int Lxf, int Lyf, int block, int quad, int dtype,

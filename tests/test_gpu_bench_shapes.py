@@ -338,12 +338,16 @@ def assert_capped(work, grid, what):
 
 
 def rel(got, want):
-    """max |got - want| / max |want| in fp64, in chunks (no full-size temporaries)."""
+    """max |got - want| / max |want| in fp64, in chunks (no full-size temporaries); NaN when either side holds a NaN
+    (Python's max() would silently drop it)."""
     g, w = got.reshape(-1), want.reshape(-1)
     num = den = 0.0
     for i in range(0, w.numel(), 1 << 24):
         wi = w[i:i + (1 << 24)].to(torch.complex128)
-        num = max(num, float((g[i:i + (1 << 24)].to(torch.complex128) - wi).abs().max()))
+        d = float((g[i:i + (1 << 24)].to(torch.complex128) - wi).abs().max())
+        if math.isnan(d):
+            return math.nan
+        num = max(num, d)
         den = max(den, float(wi.abs().max()))
     return num / max(den, 1e-300)
 
