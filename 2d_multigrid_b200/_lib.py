@@ -25,6 +25,10 @@ SIGNATURES = {
     "mg2d_wilson_sw_relax_rb": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _d, _i, _i, _i, _i, _i, _vp],
     "mg2d_wilson_sw_relax_rb2": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _d, _i, _i, _i, _i, _vp, _vp],
     "mg2d_clover_add": [_vp, _vp, _ll, _i, _vp],
+    "mg2d_wilson_tm_apply": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _i, _i, _i, _vp, _vp],
+    "mg2d_wilson_tm_relax_rb": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _i, _i, _i, _i, _vp],
+    "mg2d_wilson_tm_relax_rb2": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _i, _i, _i, _vp, _vp],
+    "mg2d_twist_add": [_vp, _d, _ll, _i, _vp],
     "mg2d_stencil_apply": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _ll, _ll, _vp, _vp],
     "mg2d_block_inverse": [_vp, _vp, _i, _ll, _i, _vp],
     "mg2d_relax_jacobi": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _ll, _ll, _vp],

@@ -6,7 +6,8 @@ x <- D(m_k)^-1 x, each solve done by the MG-preconditioned FGCR; the shift moves
 (a new hierarchy per stage), and the eigenvalue is read off the gamma5-symmetric quotient
     lambda ~ <g5 x, D(0) x> / <g5 x, x>        (D is gamma5-hermitian, so g5 x is the LEFT eigenvector: second-order accurate;
                                                  falls back to the plain Rayleigh quotient when <g5 x, x> ~ 0)
-Input preparation, not part of the timed hot path.
+Input preparation, not part of the timed hot path.  The operator must be untwisted (mu == 0): the twisted-mass solve at
+maximal twist takes the m_crit found here.
 """
 from __future__ import annotations
 
@@ -27,6 +28,13 @@ def _quotients(x, Dx, wilson: bool):
     return (torch.vdot(g5x.reshape(-1), Df) / den).item(), rq
 
 
+def _untwisted(p):
+    if getattr(p, "mu", 0.0) != 0.0:
+        raise ValueError("estimate_critical_mass needs mu == 0: the gamma5 quotient relies on gamma5-hermiticity, which the "
+                         "twisted mass breaks; estimate m_crit at mu = 0 and pass it to the twisted solve")
+    return p
+
+
 def estimate_critical_mass(U, params_factory, m0: float = 0.0, iters: int = 4, refine: int = 3, tol: float = 1e-8,
                            margins=(0.02, 0.004), target: float = 2e-5, max_refine: int = 12, verbose: bool = False):
     """params_factory(mass) -> MGParams.  Returns (m_crit_estimate, history of eigenvalue estimates of D(0)).
@@ -39,10 +47,11 @@ def estimate_critical_mass(U, params_factory, m0: float = 0.0, iters: int = 4, r
     lam = None
     nsolves = 0
     stages = [(m0, iters, iters)] + [(None, refine, max_refine)] * len(margins)
+    _untwisted(params_factory(m0))
     for stage, (m, nmin, nmax) in enumerate(stages):
         if m is None:
             m = -lam.real + margins[stage - 1]
-        p = params_factory(m)
+        p = _untwisted(params_factory(m))
         mg = setup(U, p, init="device")
         lv = mg.LVL[0]
         wilson = p.stencil == "wilson"

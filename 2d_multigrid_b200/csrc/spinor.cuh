@@ -51,4 +51,28 @@ __device__ __forceinline__ void store_spinor(cplx<T>* __restrict__ p, size_t s, 
     }
 }
 
+// Twisted mass (template flag TM of the Wilson kernels): self block diag(d+f+i mu, d-f-i mu), d = 2+m, f the clover field
+// (0 without clover).  A sweep multiplies component 0 by z0 = 1/(d+f+i mu) and component 1 by z1 = 1/(d-f-i mu).  Where
+// f == 0 these are the launch constants tz = 1/(d+i mu) and conj(tz); a clover site takes both from one reciprocal
+// 1/(|d+f+i mu|^2 |d-f-i mu|^2).
+template <typename T>
+__device__ __forceinline__ void tm_self_inverse(T f, T d, T mu, cplx<T> tz, cplx<T>& z0, cplx<T>& z1) {
+    z0 = tz; z1 = cconj(tz);
+    if (f != (T)0) {
+        const T a = d + f, b = d - f, mu2 = mu * mu;
+        const T na = fma(a, a, mu2), nb = fma(b, b, mu2);
+        const T q = (T)1 / (na * nb);
+        const T ia = nb * q, ib = na * q;                   // 1/|a+i mu|^2, 1/|b-i mu|^2
+        z0 = mk<T>(a * ia, -mu * ia);
+        z1 = mk<T>(b * ib, mu * ib);
+    }
+}
+// the launch constant tz = 1/(d + i mu) of tm_self_inverse, formed in double on the host
+template <typename T>
+inline cplx<T> tm_tz(double d, double mu) {
+    const double den = d * d + mu * mu;
+    cplx<T> z; z.x = (T)(d / den); z.y = (T)(-mu / den);
+    return z;
+}
+
 }  // namespace

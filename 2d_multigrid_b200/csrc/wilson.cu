@@ -11,6 +11,9 @@
 // Clover (Sheikholeslami-Wohlert) variant, template flag SW: the self term becomes (2+m) 1 + f(s) s3 with the real site field
 // f of mg2d_clover_field (csrc/gauge.cu), i.e. (2+m+f) on component 0 and (2+m-f) on component 1.
 //
+// Twisted-mass variant, template flag TM (with or without SW): + i mu gamma5 = i mu s3 on the self term, i.e. (2+m+f+i mu) on
+// component 0 and (2+m-f-i mu) on component 1.  mu is one constant per launch, so the bytes are those of the Wilson / SW kernel.
+//
 // HBM roofline: algorithmic traffic 96 B/site in complex128 (psi in 32 + links 32 + out 32), +32 with b; SW adds f: 104 B/site
 // (c64: 48 -> 52).
 //
@@ -19,6 +22,7 @@
 // psi/U element is loaded from global memory exactly once per CTA (plus the two halo rows of the march and
 // two halo columns); x-neighbour data is exchanged as projected half-spinors (one complex each way) through
 // warp shuffles, with the warp-edge lanes falling back to a global load.
+#include <cmath>
 #include "common.cuh"
 #include "spinor.cuh"
 
@@ -34,16 +38,20 @@ inline int mg2d_fail2(mg2d_ctx* ctx, const char* name, const char* what) {
 }
 
 // MODE 0: out = D in ; MODE 1: out = b - D in.  DOTS: also reduce |out|^2, <out,in>, |b|^2.  SW: clover self term from F.
-// (the clover variants with DOTS ask for 5 CTAs per SM: left to its own heuristic ptxas spills the loop bound of the complex128
-// residual-norm variant; the Wilson instantiations keep the plain bound and their code)
-template <typename T, int MODE, bool DOTS, bool SW>
-__global__ void __launch_bounds__(WX, (SW && DOTS) ? 5 : 0)
+// TM: twisted-mass self term i mu s3.
+// (the clover and twisted variants with DOTS ask for 5 CTAs per SM: left to its own heuristic ptxas spills the loop bound of
+// the complex128 residual-norm variant.  The twisted variants without DOTS ask for the occupancy the Wilson kernel reaches,
+// 7 CTAs per SM in complex128 (72 registers) and 10 in complex64 (48): left alone, ptxas gives the complex128 twisted apply
+// 78 registers, 6 CTAs per SM, and it runs 24% slower than the Wilson apply.  The Wilson instantiations keep the plain bound
+// and their code)
+template <typename T, int MODE, bool DOTS, bool SW, bool TM>
+__global__ void __launch_bounds__(WX, ((SW || TM) && DOTS) ? 5 : (TM ? (sizeof(T) == 8 ? 7 : 10) : 0))
 wilson_march_kernel(cplx<T>* __restrict__ out, const cplx<T>* __restrict__ in,
                     const cplx<T>* __restrict__ in_lo, const cplx<T>* __restrict__ in_hi,
                     const cplx<T>* __restrict__ U, const cplx<T>* __restrict__ U_lo,
                     const cplx<T>* __restrict__ b, T diag, int Lx, int Ly, int RY,
                     double* __restrict__ partials, unsigned int* __restrict__ counter,
-                    double* __restrict__ dots, XComm* xc, const T* __restrict__ F) {
+                    double* __restrict__ dots, XComm* xc, const T* __restrict__ F, T mu) {
     using C = cplx<T>;
     const int nsx = (Lx + WX - 1) / WX;
     const int nsy = (Ly + RY - 1) / RY;
@@ -102,6 +110,10 @@ wilson_march_kernel(cplx<T>* __restrict__ out, const cplx<T>* __restrict__ in,
                 o.c0.x = fma(f, cur.c0.x, o.c0.x); o.c0.y = fma(f, cur.c0.y, o.c0.y);
                 o.c1.x = fma(-f, cur.c1.x, o.c1.x); o.c1.y = fma(-f, cur.c1.y, o.c1.y);
             }
+            if (TM) {                                             // + i mu s3 psi(s)
+                o.c0.x = fma(-mu, cur.c0.y, o.c0.x); o.c0.y = fma(mu, cur.c0.x, o.c0.y);
+                o.c1.x = fma(mu, cur.c1.y, o.c1.x); o.c1.y = fma(-mu, cur.c1.x, o.c1.y);
+            }
             if (MODE == 1) {
                 Spinor<T> bb = load_spinor<T>(b, s);
                 if (DOTS && active) red[3] += (double)bb.c0.x * bb.c0.x + (double)bb.c0.y * bb.c0.y
@@ -131,11 +143,12 @@ wilson_march_kernel(cplx<T>* __restrict__ out, const cplx<T>* __restrict__ in,
 // updated site; a warp covers 64 consecutive x.  Traffic per full sweep (c128): phi 32+32, r 32, links 2x32; SW: + f 8.
 // SW: D0 = diag(d+f, d-f), d = 2+m, inverted from one reciprocal 1/((d+f)(d-f)); a site with f == 0 uses inv_diag itself,
 // so c_sw = 0 reproduces the Wilson sweep bit for bit.
-template <typename T, bool SW>
+// TM: D0 = diag(d+f+i mu, d-f-i mu) (f = 0 without SW), inverted by tm_self_inverse (spinor.cuh), tz = 1/(d+i mu).
+template <typename T, bool SW, bool TM>
 __global__ void __launch_bounds__(256)
 wilson_rb_kernel(cplx<T>* phi, const cplx<T>* lo, const cplx<T>* hi, const cplx<T>* __restrict__ U,
                  const cplx<T>* __restrict__ U_lo, const cplx<T>* __restrict__ r, T inv_diag, int Lx, int Ly,
-                 int colour, int yoff, const T* __restrict__ F, T diag) {
+                 int colour, int yoff, const T* __restrict__ F, T diag, T mu, cplx<T> tz) {
     using C = cplx<T>;
     const int Lh = Lx / 2;
     const long long S2 = (long long)Lh * Ly;
@@ -158,12 +171,18 @@ wilson_rb_kernel(cplx<T>* phi, const cplx<T>* lo, const cplx<T>* hi, const cplx<
         const C h0 = cadd(cadd(A, B), cadd(Cc, Dd));
         const C h1 = cadd(csub(B, A), cmul_i(csub(Dd, Cc)));
         T i0 = inv_diag, i1 = inv_diag;
-        if (SW) {
+        if (SW && !TM) {
             const T f = __ldg(F + s);
             if (f != (T)0) { const T q = (T)1 / ((diag + f) * (diag - f)); i0 = (diag - f) * q; i1 = (diag + f) * q; }
         }
         Spinor<T> o;
-        if (r) {
+        if (TM) {
+            C z0, z1;
+            tm_self_inverse<T>(SW ? __ldg(F + s) : (T)0, diag, mu, tz, z0, z1);
+            C t0 = mk<T>(-half * h0.x, -half * h0.y), t1 = mk<T>(-half * h1.x, -half * h1.y);
+            if (r) { const Spinor<T> rr = load_spinor<T>(r, s); t0 = cadd(rr.c0, t0); t1 = cadd(rr.c1, t1); }
+            o.c0 = cmul(t0, z0); o.c1 = cmul(t1, z1);
+        } else if (r) {
             const Spinor<T> rr = load_spinor<T>(r, s);
             o.c0.x = (rr.c0.x - half * h0.x) * i0; o.c0.y = (rr.c0.y - half * h0.y) * i0;
             o.c1.x = (rr.c1.x - half * h1.x) * i1; o.c1.y = (rr.c1.y - half * h1.y) * i1;
@@ -221,10 +240,19 @@ __global__ void clover_add_kernel(cplx<T>* __restrict__ D, const T* __restrict__
     }
 }
 
+// twisted-mass term of the stored level-0 Wilson operator: D[s][0] += diag(i mu, -i mu)
+template <typename T>
+__global__ void twist_add_kernel(cplx<T>* __restrict__ D, T mu, long long S) {
+    for (long long s = blockIdx.x * (long long)blockDim.x + threadIdx.x; s < S; s += (long long)gridDim.x * blockDim.x) {
+        D[20 * s].y += mu;
+        D[20 * s + 3].y -= mu;
+    }
+}
+
 template <typename T>
 int launch_wilson(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo, const void* in_hi, const void* U,
-                  const void* U_lo, const void* F, const void* b, double mass, int Lx, int Ly, int mode, double* dots,
-                  cudaStream_t st, const char* name) {
+                  const void* U_lo, const void* F, const void* b, double mass, bool tm, double mu, int Lx, int Ly, int mode,
+                  double* dots, cudaStream_t st, const char* name) {
     using C = cplx<T>;
     // rows per work item: as many as possible (each item re-reads 2 halo rows) while >= 6 CTAs per SM exist
     int RY = RY_MAX;
@@ -232,38 +260,40 @@ int launch_wilson(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo, c
     const int nwork = ((Lx + WX - 1) / WX) * ((Ly + RY - 1) / RY);
     int grid = nwork < MG2D_MAX_PARTIALS ? nwork : MG2D_MAX_PARTIALS;
     const T diag = (T)(2.0 + mass);
-#define WL(MODE, DOTS, SW)                                                                                  \
-    wilson_march_kernel<T, MODE, DOTS, SW><<<grid, WX, 0, st>>>((C*)out, (const C*)in, (const C*)in_lo,      \
+#define WL(MODE, DOTS, SW, TM)                                                                              \
+    wilson_march_kernel<T, MODE, DOTS, SW, TM><<<grid, WX, 0, st>>>((C*)out, (const C*)in, (const C*)in_lo,  \
         (const C*)in_hi, (const C*)U, (const C*)U_lo, (const C*)b, diag, Lx, Ly, RY, ctx->partials, ctx->counter, dots, \
-        ctx->xreduce ? ctx->xcomm : nullptr, (const T*)F)
-    if (F) {
-        if (mode == MG2D_MODE_APPLY) { if (dots) WL(0, true, true); else WL(0, false, true); }
-        else                         { if (dots) WL(1, true, true); else WL(1, false, true); }
+        ctx->xreduce ? ctx->xcomm : nullptr, (const T*)F, (T)mu)
+#define WL_MODES(SW, TM)                                                                                    \
+    if (mode == MG2D_MODE_APPLY) { if (dots) WL(0, true, SW, TM); else WL(0, false, SW, TM); }              \
+    else                         { if (dots) WL(1, true, SW, TM); else WL(1, false, SW, TM); }
+    if (tm) {
+        if (F) { WL_MODES(true, true) } else { WL_MODES(false, true) }
     } else {
-        if (mode == MG2D_MODE_APPLY) { if (dots) WL(0, true, false); else WL(0, false, false); }
-        else                         { if (dots) WL(1, true, false); else WL(1, false, false); }
+        if (F) { WL_MODES(true, false) } else { WL_MODES(false, false) }
     }
+#undef WL_MODES
 #undef WL
     return mg2d_check_launch(ctx, name);
 }
 
 int wilson_apply(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo, const void* in_hi, const void* U, const void* U_lo,
-                 const void* F, const void* b, double mass, int Lx, int Ly, int mode, int dtype, double* dots, void* stream,
-                 const char* name) {
+                 const void* F, const void* b, double mass, bool tm, double mu, int Lx, int Ly, int mode, int dtype, double* dots,
+                 void* stream, const char* name) {
     if (!ctx) return MG2D_EINVAL;
     if (!out || !in || !in_lo || !in_hi || !U || !U_lo || Lx < 2 || Ly < 1) return mg2d_fail2(ctx, name, "bad argument");
     if (mode == MG2D_MODE_RESID && !b) return mg2d_fail2(ctx, name, "MODE_RESID needs b");
     if (mode != MG2D_MODE_APPLY && mode != MG2D_MODE_RESID) return mg2d_fail2(ctx, name, "bad mode");
     if (out == in) return mg2d_fail2(ctx, name, "out must not alias in");
     cudaStream_t st = (cudaStream_t)stream;
-    if (dtype == MG2D_C128) return launch_wilson<double>(ctx, out, in, in_lo, in_hi, U, U_lo, F, b, mass, Lx, Ly, mode, dots, st, name);
-    if (dtype == MG2D_C64)  return launch_wilson<float>(ctx, out, in, in_lo, in_hi, U, U_lo, F, b, mass, Lx, Ly, mode, dots, st, name);
+    if (dtype == MG2D_C128) return launch_wilson<double>(ctx, out, in, in_lo, in_hi, U, U_lo, F, b, mass, tm, mu, Lx, Ly, mode, dots, st, name);
+    if (dtype == MG2D_C64)  return launch_wilson<float>(ctx, out, in, in_lo, in_hi, U, U_lo, F, b, mass, tm, mu, Lx, Ly, mode, dots, st, name);
     return mg2d_fail2(ctx, name, "bad dtype");
 }
 
 int wilson_relax_rb(mg2d_ctx* ctx, void* phi, const void* phi_lo, const void* phi_hi, const void* U, const void* U_lo,
-                    const void* F, const void* r, double mass, int Lx, int Ly, int colour, int yoff, int dtype, void* stream,
-                    const char* name) {
+                    const void* F, const void* r, double mass, bool tm, double mu, int Lx, int Ly, int colour, int yoff, int dtype,
+                    void* stream, const char* name) {
     if (!ctx) return MG2D_EINVAL;
     if (!phi || !phi_lo || !phi_hi || !U || !U_lo || Lx < 2 || (Lx & 1) || Ly < 1 || (colour != 0 && colour != 1))
         return mg2d_fail2(ctx, name, "bad argument (Lx must be even)");
@@ -271,11 +301,14 @@ int wilson_relax_rb(mg2d_ctx* ctx, void* phi, const void* phi_lo, const void* ph
     const long long S2 = (long long)(Lx / 2) * Ly;
     long long nb = (S2 + 255) / 256; if (nb > (long long)ctx->num_sms * 32) nb = (long long)ctx->num_sms * 32;
     const double inv = 1.0 / (2.0 + mass);
-#define RB(T, SW) wilson_rb_kernel<T, SW><<<(int)nb, 256, 0, st>>>((cplx<T>*)phi, (const cplx<T>*)phi_lo, (const cplx<T>*)phi_hi,  \
-        (const cplx<T>*)U, (const cplx<T>*)U_lo, (const cplx<T>*)r, (T)inv, Lx, Ly, colour, yoff, (const T*)F, (T)(2.0 + mass))
-    if (dtype == MG2D_C128) { if (F) RB(double, true); else RB(double, false); }
-    else if (dtype == MG2D_C64) { if (F) RB(float, true); else RB(float, false); }
+#define RB(T, SW, TM) wilson_rb_kernel<T, SW, TM><<<(int)nb, 256, 0, st>>>((cplx<T>*)phi, (const cplx<T>*)phi_lo,   \
+        (const cplx<T>*)phi_hi, (const cplx<T>*)U, (const cplx<T>*)U_lo, (const cplx<T>*)r, (T)inv, Lx, Ly, colour, yoff,  \
+        (const T*)F, (T)(2.0 + mass), (T)mu, tm_tz<T>(2.0 + mass, mu))
+#define RB_SW(T, TM) { if (F) RB(T, true, TM); else RB(T, false, TM); }
+    if (dtype == MG2D_C128) { if (tm) RB_SW(double, true) else RB_SW(double, false) }
+    else if (dtype == MG2D_C64) { if (tm) RB_SW(float, true) else RB_SW(float, false) }
     else return mg2d_fail2(ctx, name, "bad dtype");
+#undef RB_SW
 #undef RB
     return mg2d_check_launch(ctx, name);
 }
@@ -285,14 +318,24 @@ int wilson_relax_rb(mg2d_ctx* ctx, void* phi, const void* phi_lo, const void* ph
 extern "C" int mg2d_wilson_apply(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo, const void* in_hi,
                                  const void* U, const void* U_lo, const void* b, double mass, int Lx, int Ly,
                                  int mode, int dtype, double* dots, void* stream) {
-    return wilson_apply(ctx, out, in, in_lo, in_hi, U, U_lo, nullptr, b, mass, Lx, Ly, mode, dtype, dots, stream, "mg2d_wilson_apply");
+    return wilson_apply(ctx, out, in, in_lo, in_hi, U, U_lo, nullptr, b, mass, false, 0.0, Lx, Ly, mode, dtype, dots, stream,
+                        "mg2d_wilson_apply");
 }
 
 extern "C" int mg2d_wilson_sw_apply(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo, const void* in_hi,
                                     const void* U, const void* U_lo, const void* F, const void* b, double mass, int Lx, int Ly,
                                     int mode, int dtype, double* dots, void* stream) {
     if (ctx && !F) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_sw_apply: F is NULL");
-    return wilson_apply(ctx, out, in, in_lo, in_hi, U, U_lo, F, b, mass, Lx, Ly, mode, dtype, dots, stream, "mg2d_wilson_sw_apply");
+    return wilson_apply(ctx, out, in, in_lo, in_hi, U, U_lo, F, b, mass, false, 0.0, Lx, Ly, mode, dtype, dots, stream,
+                        "mg2d_wilson_sw_apply");
+}
+
+extern "C" int mg2d_wilson_tm_apply(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo, const void* in_hi,
+                                    const void* U, const void* U_lo, const void* F, const void* b, double mass, double mu, int Lx,
+                                    int Ly, int mode, int dtype, double* dots, void* stream) {
+    if (ctx && !std::isfinite(mu)) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_tm_apply: mu is not finite");
+    return wilson_apply(ctx, out, in, in_lo, in_hi, U, U_lo, F, b, mass, true, mu, Lx, Ly, mode, dtype, dots, stream,
+                        "mg2d_wilson_tm_apply");
 }
 
 extern "C" int mg2d_lvl0_matrix(mg2d_ctx* ctx, void* D, const void* U, const void* U_lo, double mass, int stencil,
@@ -321,15 +364,36 @@ extern "C" int mg2d_clover_add(mg2d_ctx* ctx, void* D, const void* F, long long 
     return mg2d_check_launch(ctx, "mg2d_clover_add");
 }
 
+extern "C" int mg2d_twist_add(mg2d_ctx* ctx, void* D, double mu, long long nsites, int dtype, void* stream) {
+    if (!ctx) return MG2D_EINVAL;
+    if (!D || nsites < 1 || !std::isfinite(mu)) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_twist_add: bad argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    long long grid = (nsites + 255) / 256; if (grid > (long long)ctx->num_sms * 8) grid = (long long)ctx->num_sms * 8;
+    if (dtype == MG2D_C128) twist_add_kernel<double><<<(int)grid, 256, 0, st>>>((double2*)D, mu, nsites);
+    else if (dtype == MG2D_C64) twist_add_kernel<float><<<(int)grid, 256, 0, st>>>((float2*)D, (float)mu, nsites);
+    else return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_twist_add: bad dtype");
+    return mg2d_check_launch(ctx, "mg2d_twist_add");
+}
+
 extern "C" int mg2d_wilson_relax_rb(mg2d_ctx* ctx, void* phi, const void* phi_lo, const void* phi_hi, const void* U,
                                     const void* U_lo, const void* r, double mass, int Lx, int Ly, int colour, int yoff,
                                     int dtype, void* stream) {
-    return wilson_relax_rb(ctx, phi, phi_lo, phi_hi, U, U_lo, nullptr, r, mass, Lx, Ly, colour, yoff, dtype, stream, "mg2d_wilson_relax_rb");
+    return wilson_relax_rb(ctx, phi, phi_lo, phi_hi, U, U_lo, nullptr, r, mass, false, 0.0, Lx, Ly, colour, yoff, dtype, stream,
+                           "mg2d_wilson_relax_rb");
 }
 
 extern "C" int mg2d_wilson_sw_relax_rb(mg2d_ctx* ctx, void* phi, const void* phi_lo, const void* phi_hi, const void* U,
                                        const void* U_lo, const void* F, const void* r, double mass, int Lx, int Ly, int colour,
                                        int yoff, int dtype, void* stream) {
     if (ctx && !F) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_sw_relax_rb: F is NULL");
-    return wilson_relax_rb(ctx, phi, phi_lo, phi_hi, U, U_lo, F, r, mass, Lx, Ly, colour, yoff, dtype, stream, "mg2d_wilson_sw_relax_rb");
+    return wilson_relax_rb(ctx, phi, phi_lo, phi_hi, U, U_lo, F, r, mass, false, 0.0, Lx, Ly, colour, yoff, dtype, stream,
+                           "mg2d_wilson_sw_relax_rb");
+}
+
+extern "C" int mg2d_wilson_tm_relax_rb(mg2d_ctx* ctx, void* phi, const void* phi_lo, const void* phi_hi, const void* U,
+                                       const void* U_lo, const void* F, const void* r, double mass, double mu, int Lx, int Ly,
+                                       int colour, int yoff, int dtype, void* stream) {
+    if (ctx && !std::isfinite(mu)) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_wilson_tm_relax_rb: mu is not finite");
+    return wilson_relax_rb(ctx, phi, phi_lo, phi_hi, U, U_lo, F, r, mass, true, mu, Lx, Ly, colour, yoff, dtype, stream,
+                           "mg2d_wilson_tm_relax_rb");
 }

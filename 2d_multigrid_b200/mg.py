@@ -198,6 +198,9 @@ class Level:
                         0 if p.stencil == "wilson" else 1, self.L, self.Ly, mg.dcode, _stream())
             if self.clover is not None:
                 mg.ctx.call("mg2d_clover_add", _ptr(self.D), _ptr(self.clover), self.S, mg.dcode, _stream())
+            if p.mu != 0.0:
+                # twisted mass: + i mu sigma3 on the self blocks; the Galerkin products carry it to every coarse level
+                mg.ctx.call("mg2d_twist_add", _ptr(self.D), float(p.mu), self.S, mg.dcode, _stream())
             self.D0inv = None
             self.M = None
         self.matrix_free = not store
@@ -245,7 +248,10 @@ class Level:
                                   None if dots is None else dots[4 * v:], 1)
                 return
             lo, hi = self._halo(vin)
-            if self.clover is None:
+            if mg.p.mu != 0.0:
+                mg.ctx.call("mg2d_wilson_tm_apply", _ptr(out), _ptr(vin), lo, hi, _ptr(self.U), self.U_lo_ptr, _ptr(self.clover),
+                            _ptr(b), float(mg.p.mass), float(mg.p.mu), self.L, self.Ly, mode, mg.dcode, _ptr(dots), _stream())
+            elif self.clover is None:
                 mg.ctx.call("mg2d_wilson_apply", _ptr(out), _ptr(vin), lo, hi, _ptr(self.U), self.U_lo_ptr, _ptr(b),
                             float(mg.p.mass), self.L, self.Ly, mode, mg.dcode, _ptr(dots), _stream())
             else:
@@ -405,7 +411,12 @@ class Level:
                         link = ctypes.byref(lk)
                     else:
                         lo2, hi2 = self._halo(cur, depth=2)
-                    if self.clover is None:
+                    if mg.p.mu != 0.0:
+                        F_lo, F_hi = (None, None) if self.clover is None else (self.clover_lo_ptr, self.clover_hi_ptr)
+                        mg.ctx.call("mg2d_wilson_tm_relax_rb2", _ptr(nxt), _ptr(cur), lo2, hi2, _ptr(self.U), self.U_lo2_ptr,
+                                    self.U_hi_ptr, _ptr(self.clover), F_lo, F_hi, _ptr(rv), r_lo, r_hi, float(mg.p.mass),
+                                    float(mg.p.mu), self.L, self.Ly, self.y0 & 1, mg.dcode, link, _stream())
+                    elif self.clover is None:
                         mg.ctx.call("mg2d_wilson_relax_rb2", _ptr(nxt), _ptr(cur), lo2, hi2, _ptr(self.U), self.U_lo2_ptr,
                                     self.U_hi_ptr, _ptr(rv), r_lo, r_hi, float(mg.p.mass), self.L, self.Ly, self.y0 & 1,
                                     mg.dcode, link, _stream())
@@ -432,7 +443,11 @@ class Level:
                             ph = phi if nvec == 1 else phi[v]
                             rv = None if r is None else (r if nvec == 1 else r[v])
                             lo, hi = self._halo(ph)
-                            if self.clover is None:
+                            if mg.p.mu != 0.0:
+                                mg.ctx.call("mg2d_wilson_tm_relax_rb", _ptr(ph), lo, hi, _ptr(self.U), self.U_lo_ptr,
+                                            _ptr(self.clover), _ptr(rv), float(mg.p.mass), float(mg.p.mu), self.L, self.Ly, colour,
+                                            self.y0 & 1, mg.dcode, _stream())
+                            elif self.clover is None:
                                 mg.ctx.call("mg2d_wilson_relax_rb", _ptr(ph), lo, hi, _ptr(self.U), self.U_lo_ptr, _ptr(rv),
                                             float(mg.p.mass), self.L, self.Ly, colour, self.y0 & 1, mg.dcode, _stream())
                             else:

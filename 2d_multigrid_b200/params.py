@@ -47,6 +47,8 @@ class MGParams:
                                      # default: True for smoother 'mr', False for 'gs'/'jacobi' (they need D0)
     csw: float = 0.0                 # clover (Sheikholeslami-Wohlert) coefficient of the level-0 Wilson operator: self block
                                      # (2+m) 1 + f(s) sigma3, f(s) = (csw/8) sum of Im U_P over the 4 plaquettes at s; 1 = tree level
+    mu: float = 0.0                  # twisted mass of the level-0 Wilson(-clover) operator: + i mu gamma5 = i mu sigma3 on the self
+                                     # block, so D^dag D gains mu^2 and no singular value is below |mu| (solvable at m = m_crit)
     size: list = field(default_factory=list)
     n_dof: list = field(default_factory=list)
 
@@ -103,6 +105,11 @@ class MGParams:
         if self.csw != 0.0 and not 2.0 + self.mass - abs(self.csw) / 2.0 > 0.0:
             # |f| <= |csw|/2, so this bound keeps every clover self block diag(2+m+f, 2+m-f) invertible
             raise ValueError(f"clover self blocks may be singular: need 2 + mass - |csw|/2 > 0 (mass {self.mass}, csw {self.csw})")
+        self.mu = float(self.mu)
+        if not math.isfinite(self.mu):
+            raise ValueError(f"the twisted mass must be finite (mu {self.mu})")
+        if self.mu != 0.0 and self.stencil != "wilson":
+            raise ValueError("the twisted mass (mu != 0) exists for stencil='wilson' only")
 
     @property
     def diag(self) -> float:

@@ -82,6 +82,25 @@ int mg2d_wilson_sw_relax_rb2(mg2d_ctx*, void* out, const void* in, const void* i
                              const void* F_hi, const void* r, const void* r_lo, const void* r_hi, double mass, int Lx,
                              int Ly, int yoff, int dtype, const struct mg2d_halo_link* link, void* stream);
 int mg2d_clover_add(mg2d_ctx*, void* D, const void* F, long long nsites, int dtype, void* stream);
+/* Twisted mass: + i mu gamma5 = i mu s3 on the level-0 self block, which becomes diag(2+m+f+i mu, 2+m-f-i mu) with f the
+ * clover field (F == NULL: no clover, f = 0).  D_tm^dag D_tm = D^dag D + mu^2, and g5 D_tm(mu) g5 = D_tm(-mu)^dag.
+ *   mg2d_wilson_tm_apply       mg2d_wilson_sw_apply with the twisted self term (APPLY, RESID, fused dots)
+ *   mg2d_wilson_tm_relax_rb    mg2d_wilson_sw_relax_rb with D0 = diag(2+m+f+i mu, 2+m-f-i mu)
+ *   mg2d_wilson_tm_relax_rb2   mg2d_wilson_sw_relax_rb2 with the same D0 (F, F_lo, F_hi all NULL or F_lo / F_hi given)
+ *   mg2d_twist_add             stored operator: D[s][0] += diag(i mu, -i mu) on nsites sites (stencil 0 blocks)
+ * mu must be finite.  The coarse levels need no entry point: on a chirality-split projector the Galerkin product carries
+ * the twist as i mu Gamma5_c on the coarse self blocks. */
+int mg2d_wilson_tm_apply(mg2d_ctx*, void* out, const void* in, const void* in_lo, const void* in_hi,
+                         const void* U, const void* U_lo, const void* F, const void* b, double mass, double mu, int Lx,
+                         int Ly, int mode, int dtype, double* dots, void* stream);
+int mg2d_wilson_tm_relax_rb(mg2d_ctx*, void* phi, const void* phi_lo, const void* phi_hi, const void* U,
+                            const void* U_lo, const void* F, const void* r, double mass, double mu, int Lx, int Ly,
+                            int colour, int yoff, int dtype, void* stream);
+int mg2d_wilson_tm_relax_rb2(mg2d_ctx*, void* out, const void* in, const void* in_lo2, const void* in_hi2,
+                             const void* U, const void* U_lo2, const void* U_hi, const void* F, const void* F_lo,
+                             const void* F_hi, const void* r, const void* r_lo, const void* r_hi, double mass, double mu,
+                             int Lx, int Ly, int yoff, int dtype, const struct mg2d_halo_link* link, void* stream);
+int mg2d_twist_add(mg2d_ctx*, void* D, double mu, long long nsites, int dtype, void* stream);
 
 /* ---- generic 5-point block stencil (all coarse levels; level 0 in reference-compat mode) -------------- */
 /* Level::f_apply_D / f_residue, n in {1,2,4,8,16,32}; nvec vectors `vstride` elements apart. */
