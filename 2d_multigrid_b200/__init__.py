@@ -19,6 +19,17 @@ Public API (SURVEY.md section 8b; argument order follows the reference functions
     prolongation(vec_f, vec_c, level, mg, quad)  # Near_null::f_prolongation S6/near_null.h:242-264 (level = coarse)
     near_null(level, mg) / norm_nn(level, quad, mg) / ortho(level, quad, mg) / compute_coarse_matrix(level, quad, mg)
 
+Gauge-field updates and HMC (matrix-free complex128 Wilson hierarchies on one GPU, csw = 0):
+
+    mg.update_links(U)                           # new links copied into the hierarchy in place; captured graphs replay on them
+    mg.refresh(null_iters=0)                     # coarse hierarchy rebuilt for the current links from the current near-null
+                                                 # vectors (relaxed null_iters sweeps first); 0 = setup(U, p, null_vectors=...)
+    h = HMC(p, theta, beta, tau=1.0, n_md=10, flavours=2, seed=1, md_tol=1e-10, accept_tol=1e-12,
+            refresh_null_iters=8, precond_dtype=None, use_graph=True)
+    h.trajectory() -> dict(dH, accepted, plaquette, iters_md, iters_accept, times_ms, ...)
+                                                 # two-flavour Wilson HMC (leapfrog), fermion force from two multigrid solves;
+                                                 # flavours=0 is pure-gauge HMC; h.theta holds the phases
+
 The compute path is libmg2d_sm100.so (C ABI in include/mg2d.h) and nothing else: importing this package on a
 machine without the library is allowed (so that host logic can be tested), but creating an MG raises.
 """
@@ -32,10 +43,11 @@ from .mg import MG, Level, D_to_reference_layout, MG_simple, MG_ntl, perform_MG,
 from .params import MGParams, make_params, from_argv
 from .rng import StdMT19937
 from .scalar import ScalarMG, solve_scalar, solve_scalar_s1
+from .hmc import HMC
 
 __all__ = ["make_params", "from_argv", "MGParams", "MG", "Level", "setup", "solve", "apply_D", "residue",
            "residue_mag", "relax", "restriction", "prolongation", "near_null", "norm_nn", "ortho",
-           "compute_coarse_matrix", "run_reference_flow", "ScalarMG", "solve_scalar", "solve_scalar_s1", "gauge", "refio", "diagnostics", "MG2DError", "D_to_reference_layout"]
+           "compute_coarse_matrix", "run_reference_flow", "ScalarMG", "solve_scalar", "solve_scalar_s1", "gauge", "refio", "diagnostics", "MG2DError", "D_to_reference_layout", "HMC"]
 
 
 def apply_D(v_out, v_in, level: int, mg: MG):

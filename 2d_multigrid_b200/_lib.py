@@ -84,6 +84,10 @@ SIGNATURES = {
     "mg2d_plaquette": [_vp, _i, _i, _vp, _vp],
     "mg2d_clover_field": [_vp, _vp, _vp, _vp, _d, _i, _i, _i, _vp],
     "mg2d_phases_to_links": [_vp, _vp, _ll, _i, _vp],
+    "mg2d_fill_gaussian": [_vp, _ll, _ll, _ull, _ull, _d, _vp],
+    "mg2d_hmc_momentum": [_vp, _vp, _vp, _vp, _d, _d, _i, _vp],
+    "mg2d_hmc_links": [_vp, _vp, _d, _vp, _vp, _ll, _vp],
+    "mg2d_gamma5": [_vp, _vp, _ll, _vp],
     "mg2d_s2_relax": [_vp, _vp, _i, _d, _d, _i, _i, _vp],
     "mg2d_s2_project": [_vp, _vp, _vp, _i, _d, _d, _i, _vp],
     "mg2d_s2_interpolate": [_vp, _vp, _i, _i, _vp],

@@ -4,6 +4,7 @@
 //                          for the reference's sequential std::mt19937 stream: a COUNTER-based generator keyed on
 //                          (seed, stream, global element index), so that a strip of a domain-decomposed field holds
 //                          exactly the numbers the single-GPU field holds at the same global sites
+//   mg2d_fill_gaussian     normal deviates by Box-Muller on the same counter generator (HMC momenta and pseudofermion sources)
 //   mg2d_gauge_metropolis  one checkerboard half-update of the compact-U(1) Wilson action (the reference only reads
 //                          such configurations, S6/gauge.h:44,88-110, beta in {6, 32}); mirrored draw-for-draw by
 //                          oracle gauge_quenched_phases_counter
@@ -29,6 +30,18 @@ __global__ void fill_uniform_kernel(cplx<T>* __restrict__ out, long long n, unsi
     for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
         const double u = counter_u01(seed, stream, offset + (unsigned long long)e);
         out[e] = mk<T>((T)__dadd_rn(lo, __dmul_rn(hi - lo, u)), (T)0);     // no FMA contraction: equals the numpy oracle bit for bit
+    }
+}
+
+// out[e] = sd sqrt(-2 ln(1 - u1)) cos(2 pi u2), u1 / u2 = counter numbers at index 2(offset+e) / 2(offset+e)+1 (Box-Muller,
+// cosine branch): one real N(0, sd^2) deviate per element, so a sub-range of the field is drawn independently.
+// oracle mirror: tests/test_hmc.py counter_gaussian
+__global__ void fill_gaussian_kernel(double* __restrict__ out, long long n, unsigned long long offset, unsigned long long seed,
+                                     unsigned long long stream, double sd) {
+    for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
+        const unsigned long long k = 2ull * (offset + (unsigned long long)e);
+        const double u1 = counter_u01(seed, stream, k), u2 = counter_u01(seed, stream, k + 1ull);
+        out[e] = sd * sqrt(-2.0 * log(1.0 - u1)) * cospi(2.0 * u2);
     }
 }
 
@@ -141,6 +154,15 @@ extern "C" int mg2d_fill_uniform(mg2d_ctx* ctx, void* out, long long nelem, long
     else if (dtype == MG2D_C64) fill_uniform_kernel<float><<<grid, 256, 0, st>>>((float2*)out, nelem, (unsigned long long)offset, seed, stream_id, lo, hi);
     else return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_fill_uniform: bad dtype");
     return mg2d_check_launch(ctx, "mg2d_fill_uniform");
+}
+
+extern "C" int mg2d_fill_gaussian(mg2d_ctx* ctx, double* out, long long nelem, long long offset, unsigned long long seed,
+                                  unsigned long long stream_id, double variance, void* stream) {
+    if (!ctx) return MG2D_EINVAL;
+    if (!out || nelem < 1 || offset < 0 || !(variance >= 0.0)) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_fill_gaussian: bad argument");
+    fill_gaussian_kernel<<<grid_for(ctx, nelem), 256, 0, (cudaStream_t)stream>>>(out, nelem, (unsigned long long)offset, seed,
+                                                                                  stream_id, sqrt(variance));
+    return mg2d_check_launch(ctx, "mg2d_fill_gaussian");
 }
 
 extern "C" int mg2d_gauge_metropolis(mg2d_ctx* ctx, double* theta, int L, double beta, double delta, int mu, int parity,

@@ -343,6 +343,21 @@ int mg2d_clover_field(mg2d_ctx*, void* F, const void* U, const void* U_lo, const
                       int dtype, void* stream);
 /* U[e] = polar(1, theta[e]) (S6/gauge.h:106) */
 int mg2d_phases_to_links(mg2d_ctx*, void* U, const double* theta, long long nelem, int dtype, void* stream);
+/* out[e] = N(0, variance) real deviates: Box-Muller (cosine branch) on the counter numbers at indices 2(offset+e) and
+ * 2(offset+e)+1 of (seed, stream_id), so a draw is reproducible from its key alone (HMC momenta and pseudofermion sources). */
+int mg2d_fill_gaussian(mg2d_ctx*, double* out, long long nelem, long long offset, unsigned long long seed,
+                       unsigned long long stream_id, double variance, void* stream);
+
+/* ---- two-flavour Wilson HMC on the links U[s][mu] = e^{i theta[s][mu]} (complex128, whole lattice, L x L) ---------- */
+/* P[s][mu] -= eps (F^g_mu(s) + F^f_mu(s)) for both directions: F^g = dS_g/dtheta of S_g = beta sum_P (1 - cos theta_P);
+ * F^f = dS_f/dtheta of S_f = phi^dag (D^dag D)^-1 phi from X = (D^dag D)^-1 phi and Y = D X (csrc/hmc.cu).  X = Y = NULL:
+ * gauge force only. */
+int mg2d_hmc_momentum(mg2d_ctx*, double* P, const void* U, const void* X, const void* Y, double beta, double eps, int L,
+                      void* stream);
+/* theta[e] += eps P[e]; U[e] = polar(1, theta[e]) (complex128) and, when U32 is not NULL, its complex64 copy. */
+int mg2d_hmc_links(mg2d_ctx*, double* theta, const double* P, double eps, void* U, void* U32, long long nelem, void* stream);
+/* out = gamma5 in = sigma3 in on nsites two-component complex128 sites (out may equal in). */
+int mg2d_gamma5(mg2d_ctx*, void* out, const void* in, long long nsites, void* stream);
 
 /* ---- real scalar Laplace geometric MG, BASELINE config 1 (S2) -------------------------------------------- */
 /* relax (S2:46-72): num_iter lexicographic GS sweeps phi = scale (sum nbrs - b a^2), wavefront order. */
