@@ -30,6 +30,13 @@ Gauge-field updates and HMC (matrix-free complex128 Wilson hierarchies on one GP
                                                  # two-flavour Wilson HMC (leapfrog), fermion force from two multigrid solves;
                                                  # flavours=0 is pure-gauge HMC; h.theta holds the phases
 
+Measurements on an ensemble (complex128 links U[L*L, 2], e.g. h.mg.LVL[0].U; one-GPU complex128 Wilson hierarchies):
+
+    topological_charge(U, L) -> float            # Q = sum_P arg U_P / 2 pi, arg in (-pi, pi]
+    wilson_loops(U, L, r_max, t_max) -> [t_max, r_max] complex   # site means of the R x T loops (r_max, t_max <= 32, < L)
+    meson_correlators(mg, site=(x0, y0), tol=1e-10) -> dict(G, pp, ap, m_eff, m_pcac, iters)   # two point-source solves
+    chiral_condensate(mg, n_noise, seed=1, tol=1e-10) -> dict(mean, stderr, values, iters)     # U(1) noise, Tr D^-1 / L^2
+
 The compute path is libmg2d_sm100.so (C ABI in include/mg2d.h) and nothing else: importing this package on a
 machine without the library is allowed (so that host logic can be tested), but creating an MG raises.
 """
@@ -44,10 +51,12 @@ from .params import MGParams, make_params, from_argv
 from .rng import StdMT19937
 from .scalar import ScalarMG, solve_scalar, solve_scalar_s1
 from .hmc import HMC
+from .measure import topological_charge, wilson_loops, meson_correlators, chiral_condensate
 
 __all__ = ["make_params", "from_argv", "MGParams", "MG", "Level", "setup", "solve", "apply_D", "residue",
            "residue_mag", "relax", "restriction", "prolongation", "near_null", "norm_nn", "ortho",
-           "compute_coarse_matrix", "run_reference_flow", "ScalarMG", "solve_scalar", "solve_scalar_s1", "gauge", "refio", "diagnostics", "MG2DError", "D_to_reference_layout", "HMC"]
+           "compute_coarse_matrix", "run_reference_flow", "ScalarMG", "solve_scalar", "solve_scalar_s1", "gauge", "refio", "diagnostics", "MG2DError", "D_to_reference_layout", "HMC",
+           "topological_charge", "wilson_loops", "meson_correlators", "chiral_condensate"]
 
 
 def apply_D(v_out, v_in, level: int, mg: MG):

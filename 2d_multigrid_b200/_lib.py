@@ -88,6 +88,9 @@ SIGNATURES = {
     "mg2d_hmc_momentum": [_vp, _vp, _vp, _vp, _d, _d, _i, _vp],
     "mg2d_hmc_links": [_vp, _vp, _d, _vp, _vp, _ll, _vp],
     "mg2d_gamma5": [_vp, _vp, _ll, _vp],
+    "mg2d_meson_contract": [_vp, _vp, _i, _vp, _vp],
+    "mg2d_topo_charge": [_vp, _i, _vp, _vp],
+    "mg2d_wilson_loops": [_vp, _i, _i, _i, _vp, _vp],
     "mg2d_s2_relax": [_vp, _vp, _i, _d, _d, _i, _i, _vp],
     "mg2d_s2_project": [_vp, _vp, _vp, _i, _d, _d, _i, _vp],
     "mg2d_s2_interpolate": [_vp, _vp, _i, _i, _vp],

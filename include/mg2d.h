@@ -359,6 +359,18 @@ int mg2d_hmc_links(mg2d_ctx*, double* theta, const double* P, double eps, void* 
 /* out = gamma5 in = sigma3 in on nsites two-component complex128 sites (out may equal in). */
 int mg2d_gamma5(mg2d_ctx*, void* out, const void* in, long long nsites, void* stream);
 
+/* ---- gauge-ensemble measurements (complex128, whole lattice, L x L; csrc/measure.cu) ------------------------------ */
+/* out[y][a][b][re, im] = G_ab(y) = sum_x tr[s_a S(x,y) s_b s3 S(x,y)^dag s3] for every row y (time), a, b = 0..3, with
+ * S_{al,be}(s) = psi_be(s)_al from the two point-source propagator columns psi_be = D^-1 e_{s0,be} ([L*L][2] each, 32-byte
+ * aligned), s0 = 1 and s1, s2, s3 = gamma_x, gamma_y, gamma5.  -G_ab is the connected correlator of the bilinears s_a, s_b. */
+int mg2d_meson_contract(mg2d_ctx*, const void* psi0, const void* psi1, int L, double* out, void* stream);
+/* out[0] = sum_P arg U_P, arg in (-pi, pi], U_P oriented as in mg2d_plaquette; the topological charge is out[0] / 2 pi. */
+int mg2d_topo_charge(mg2d_ctx*, const void* U, int L, double* out, void* stream);
+/* out[2 ((T-1) r_max + R-1) + (0, 1)] = sum_s of the product of the links around the anticlockwise R x T rectangle with base
+ * s (R links along x, T along y; W(1,1) is the plaquette sum), 1 <= R <= r_max, 1 <= T <= t_max.  Needs
+ * 1 <= r_max, t_max <= 32 and r_max, t_max < L (MG2D_EINVAL otherwise). */
+int mg2d_wilson_loops(mg2d_ctx*, const void* U, int L, int r_max, int t_max, double* out, void* stream);
+
 /* ---- real scalar Laplace geometric MG, BASELINE config 1 (S2) -------------------------------------------- */
 /* relax (S2:46-72): num_iter lexicographic GS sweeps phi = scale (sum nbrs - b a^2), wavefront order. */
 int mg2d_s2_relax(mg2d_ctx*, double* phi, const double* b, int L, double scale, double a, int num_iter,
