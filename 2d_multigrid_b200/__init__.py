@@ -29,6 +29,11 @@ Gauge-field updates and HMC (matrix-free complex128 Wilson hierarchies on one GP
     h.trajectory() -> dict(dH, accepted, plaquette, iters_md, iters_accept, times_ms, ...)
                                                  # two-flavour Wilson HMC (leapfrog), fermion force from two multigrid solves;
                                                  # flavours=0 is pure-gauge HMC; h.theta holds the phases
+                                                 # flavours=1: one-flavour RHMC (rational approximations of (D^dag D)^p,
+                                                 # multi-shift CG force); spectrum=(a, b) overrides the covered range
+    rational_approx(p, a, b, tol)                # r(x) = alpha0 + sum_k alpha_k / (x + beta_k) ~ x^p on [a, b], p = -1/2 or 1/4
+    multishift_cg(mg, rhs, shifts, tol, max_iters, weights=None) -> (X[N, L*L, 2] or sum_k weights_k x_k, info)
+                                                 # (D^dag D + shifts_k) x_k = rhs on the level-0 links of mg, all k at once
 
 Measurements on an ensemble (complex128 links U[L*L, 2], e.g. h.mg.LVL[0].U; one-GPU complex128 Wilson hierarchies):
 
@@ -51,12 +56,14 @@ from .params import MGParams, make_params, from_argv
 from .rng import StdMT19937
 from .scalar import ScalarMG, solve_scalar, solve_scalar_s1
 from .hmc import HMC
+from .rational import rational_approx
+from .rhmc import multishift_cg
 from .measure import topological_charge, wilson_loops, meson_correlators, chiral_condensate
 
 __all__ = ["make_params", "from_argv", "MGParams", "MG", "Level", "setup", "solve", "apply_D", "residue",
            "residue_mag", "relax", "restriction", "prolongation", "near_null", "norm_nn", "ortho",
            "compute_coarse_matrix", "run_reference_flow", "ScalarMG", "solve_scalar", "solve_scalar_s1", "gauge", "refio", "diagnostics", "MG2DError", "D_to_reference_layout", "HMC",
-           "topological_charge", "wilson_loops", "meson_correlators", "chiral_condensate"]
+           "rational_approx", "multishift_cg", "topological_charge", "wilson_loops", "meson_correlators", "chiral_condensate"]
 
 
 def apply_D(v_out, v_in, level: int, mg: MG):

@@ -14,6 +14,8 @@ LIB_PATH = os.path.join(_HERE, "libmg2d_sm100.so")
 C128, C64 = 0, 1
 MODE_APPLY, MODE_RESID = 0, 1
 DOT_OUT2, DOT_OUTIN_RE, DOT_OUTIN_IM, DOT_B2, NDOTS = 0, 1, 2, 3, 4
+MSC_RR, MSC_ALPHA_PREV, MSC_BETA_PREV, MSC_PP, MSC_NACT, MSC_NACT_NEXT, MSC_ITER, MSC_THRESH, MSC_SHIFTS = range(9)
+MSC_MAX_SHIFTS = 64
 
 _vp, _i, _d, _ll, _ull = C.c_void_p, C.c_int, C.c_double, C.c_longlong, C.c_ulonglong
 
@@ -88,6 +90,8 @@ SIGNATURES = {
     "mg2d_hmc_momentum": [_vp, _vp, _vp, _vp, _d, _d, _i, _vp],
     "mg2d_hmc_links": [_vp, _vp, _d, _vp, _vp, _ll, _vp],
     "mg2d_gamma5": [_vp, _vp, _ll, _vp],
+    "mg2d_msc_pass_a": [_vp, _vp, _vp, _vp, _vp, _d, _i, _ll, _vp],
+    "mg2d_msc_pass_b": [_vp, _vp, _vp, _vp, _vp, _d, _i, _ll, _vp],
     "mg2d_meson_contract": [_vp, _vp, _i, _vp, _vp],
     "mg2d_topo_charge": [_vp, _i, _vp, _vp],
     "mg2d_wilson_loops": [_vp, _i, _i, _i, _vp, _vp],

@@ -359,6 +359,26 @@ int mg2d_hmc_links(mg2d_ctx*, double* theta, const double* P, double eps, void* 
 /* out = gamma5 in = sigma3 in on nsites two-component complex128 sites (out may equal in). */
 int mg2d_gamma5(mg2d_ctx*, void* out, const void* in, long long nsites, void* stream);
 
+/* ---- multi-shift CG for (D^dag D + sigma_k) x_k = phi, all shifts at once (one-flavour RHMC; csrc/rhmc.cu) ------------- */
+/* Jegerlehner's recurrences on complex128 two-component fields of nsites sites.  The base system is the smallest shift
+ * sigma_0; the host applies the operator with mg2d_wilson_apply (t = D p_0, dots[MG2D_DOT_OUT2] = |t|^2), mg2d_gamma5 and
+ * mg2d_wilson_apply again (w = D gamma5 t, so (D^dag D) p_0 = gamma5 w).  `sc` holds the fp64 scalars on the device:
+ * the slots below, then from MG2D_MSC_SHIFTS on, for N = nshift shifts sorted ascending, s_k = sigma_k - sigma_0 [N],
+ * zeta_k [N], zeta_k of the previous iteration [N], a_k [N], b_k [N], the accumulate-mode weights w_k [N], and the Lanczos
+ * history (alpha_i, beta_i) of iteration i at 2i, 2i+1.  Start: r = p_k = phi, x_k = 0, RR = |phi|^2, PP = |phi|^2,
+ * ALPHA_PREV = 1, BETA_PREV = 0, zeta = zeta_prev = 1, NACT_NEXT = N, ITER = 0, THRESH = (tol |phi|)^2.
+ *   mg2d_msc_pass_a  r -= alpha (gamma5 w + sigma_0 p_0), alpha = RR / (dots[0] + sigma_0 PP); |r|^2 reduced in the kernel,
+ *                    whose last CTA runs the scalar recurrences and sets NACT (the shifts pass B updates) and NACT_NEXT
+ *                    (1 + the last shift whose residual |zeta_k| |r| is still above THRESH^(1/2); 0 = all converged)
+ *   mg2d_msc_pass_b  k < NACT: x_k += a_k p_k, p_k = zeta_k r + b_k p_k, X and P laid out [N][nsites][2]; with X == NULL
+ *                    and y != NULL (accumulate mode) y += sum_k w_k a_k p_k instead; PP = |p_0|^2 when sigma_0 != 0 */
+enum { MG2D_MSC_RR = 0, MG2D_MSC_ALPHA_PREV = 1, MG2D_MSC_BETA_PREV = 2, MG2D_MSC_PP = 3, MG2D_MSC_NACT = 4,
+       MG2D_MSC_NACT_NEXT = 5, MG2D_MSC_ITER = 6, MG2D_MSC_THRESH = 7, MG2D_MSC_SHIFTS = 8, MG2D_MSC_MAX_SHIFTS = 64 };
+int mg2d_msc_pass_a(mg2d_ctx*, void* r, const void* w, const void* p0, const double* dots, double* sc, double sigma0,
+                    int nshift, long long nsites, void* stream);
+int mg2d_msc_pass_b(mg2d_ctx*, void* X, void* P, void* y, const void* r, double* sc, double sigma0, int nshift,
+                    long long nsites, void* stream);
+
 /* ---- gauge-ensemble measurements (complex128, whole lattice, L x L; csrc/measure.cu) ------------------------------ */
 /* out[y][a][b][re, im] = G_ab(y) = sum_x tr[s_a S(x,y) s_b s3 S(x,y)^dag s3] for every row y (time), a, b = 0..3, with
  * S_{al,be}(s) = psi_be(s)_al from the two point-source propagator columns psi_be = D^-1 e_{s0,be} ([L*L][2] each, 32-byte
