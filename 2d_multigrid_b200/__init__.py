@@ -34,6 +34,11 @@ Gauge-field updates and HMC (matrix-free complex128 Wilson hierarchies on one GP
     rational_approx(p, a, b, tol)                # r(x) = alpha0 + sum_k alpha_k / (x + beta_k) ~ x^p on [a, b], p = -1/2 or 1/4
     multishift_cg(mg, rhs, shifts, tol, max_iters, weights=None) -> (X[N, L*L, 2] or sum_k weights_k x_k, info)
                                                  # (D^dag D + shifts_k) x_k = rhs on the level-0 links of mg, all k at once
+    mg.set_twist(mu)                             # the twisted mass of a built hierarchy changed in place (no new Galerkin
+                                                 # products; graphs are kept per twist)
+    normal_solve(mg, rhs, shifts, tol, **solve_kw) -> (X[N, L*L, 2], info)
+                                                 # the same systems by multigrid: D_tm(+sqrt s)^-1 g5 D_tm(-sqrt s)^-1 g5 rhs;
+                                                 # HMC(flavours=1, mg_poles=K) sends the K smallest MD poles through it
 
 Measurements on an ensemble (complex128 links U[L*L, 2], e.g. h.mg.LVL[0].U; one-GPU complex128 Wilson hierarchies):
 
@@ -57,13 +62,13 @@ from .rng import StdMT19937
 from .scalar import ScalarMG, solve_scalar, solve_scalar_s1
 from .hmc import HMC
 from .rational import rational_approx
-from .rhmc import multishift_cg
+from .rhmc import multishift_cg, normal_solve
 from .measure import topological_charge, wilson_loops, meson_correlators, chiral_condensate
 
 __all__ = ["make_params", "from_argv", "MGParams", "MG", "Level", "setup", "solve", "apply_D", "residue",
            "residue_mag", "relax", "restriction", "prolongation", "near_null", "norm_nn", "ortho",
            "compute_coarse_matrix", "run_reference_flow", "ScalarMG", "solve_scalar", "solve_scalar_s1", "gauge", "refio", "diagnostics", "MG2DError", "D_to_reference_layout", "HMC",
-           "rational_approx", "multishift_cg", "topological_charge", "wilson_loops", "meson_correlators", "chiral_condensate"]
+           "rational_approx", "multishift_cg", "normal_solve", "topological_charge", "wilson_loops", "meson_correlators", "chiral_condensate"]
 
 
 def apply_D(v_out, v_in, level: int, mg: MG):

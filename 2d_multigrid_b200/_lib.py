@@ -31,6 +31,7 @@ SIGNATURES = {
     "mg2d_wilson_tm_relax_rb": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _i, _i, _i, _i, _vp],
     "mg2d_wilson_tm_relax_rb2": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _i, _i, _i, _vp, _vp],
     "mg2d_twist_add": [_vp, _d, _ll, _i, _vp],
+    "mg2d_twist_set": [_vp, _vp, _d, _i, _ll, _i, _vp],
     "mg2d_stencil_apply": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _ll, _ll, _vp, _vp],
     "mg2d_block_inverse": [_vp, _vp, _i, _ll, _i, _vp],
     "mg2d_relax_jacobi": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _ll, _ll, _vp],
@@ -44,6 +45,7 @@ SIGNATURES = {
     "mg2d_relax_rb_pm_sweeps": [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp],
     "mg2d_hop_factors": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp],
     "mg2d_lowrank_pack": [_vp, _vp, _vp, _vp, _i, _i, _ll, _i, _vp],
+    "mg2d_lowrank_pack_a": [_vp, _vp, _vp, _i, _i, _ll, _i, _vp],
     "mg2d_relax_rb_lr": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _ll, _ll, _vp, _vp],
     "mg2d_relax_rb_half": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp],
     "mg2d_to_half": [_vp, _vp, _ll, _vp],

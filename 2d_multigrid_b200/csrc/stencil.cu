@@ -634,7 +634,8 @@ hop_factors_kernel(cplx<T>* __restrict__ A, cplx<T>* __restrict__ B, const cplx<
 }
 
 // F (lane-ordered factors for stencil_rb_lr_kernel) from A, B and D0^-1:  ma_q = -D0^-1 a_q,  Bc = conj(B).
-template <typename T, int N, int R>
+// WITH_B = false rewrites only the -D0^-1 A half (B unread), with the same operations as the full pack.
+template <typename T, int N, int R, bool WITH_B = true>
 __global__ void __launch_bounds__(256)
 lowrank_pack_kernel(cplx<T>* __restrict__ F, const cplx<T>* __restrict__ A, const cplx<T>* __restrict__ B,
                     const cplx<T>* __restrict__ Dinv, long long S) {
@@ -647,8 +648,10 @@ lowrank_pack_kernel(cplx<T>* __restrict__ F, const cplx<T>* __restrict__ A, cons
         const C* inv = Dinv + (size_t)s * N * N;
         C* Fs = F + (size_t)s * LR::SITE;
         for (int t = 0; t < LR::IT; ++t) {
-            const int q = lane / LR::LP, j = (lane % LR::LP) * LR::IT + t;
-            Fs[32 * t + lane] = cconj(Bs[q * N + j]);
+            if (WITH_B) {
+                const int q = lane / LR::LP, j = (lane % LR::LP) * LR::IT + t;
+                Fs[32 * t + lane] = cconj(Bs[q * N + j]);
+            }
             const int i = lane % N, q2 = t * LR::H + lane / N;
             C acc = mk<T>(0, 0);
             for (int l = 0; l < N; ++l) cfma(acc, inv[l * N + i], As[q2 * N + l]);
@@ -1387,6 +1390,23 @@ extern "C" int mg2d_lowrank_pack(mg2d_ctx* ctx, void* F, const void* A, const vo
 #undef CALL_D
 #undef CALL_F
     return mg2d_fail(ctx, MG2D_EUNSUPPORTED, "mg2d_lowrank_pack: (n, rank) must be (16,4) or (8,2)");
+}
+
+extern "C" int mg2d_lowrank_pack_a(mg2d_ctx* ctx, void* F, const void* A, const void* D0inv, int n, int rank, long long S, int dtype,
+                                   void* stream) {
+    if (!ctx) return MG2D_EINVAL;
+    if (!F || !A || !D0inv || S < 1) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_lowrank_pack_a: bad argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    long long nb = (S + 7) / 8;
+    if (nb > (long long)ctx->num_sms * 16) nb = (long long)ctx->num_sms * 16;
+#define CALL_D(N, R) { lowrank_pack_kernel<double, N, R, false><<<(int)nb, 256, 0, st>>>((cplx<double>*)F, (const cplx<double>*)A, nullptr, (const cplx<double>*)D0inv, S); return mg2d_check_launch(ctx, "mg2d_lowrank_pack_a"); }
+#define CALL_F(N, R) { lowrank_pack_kernel<float, N, R, false><<<(int)nb, 256, 0, st>>>((cplx<float>*)F, (const cplx<float>*)A, nullptr, (const cplx<float>*)D0inv, S); return mg2d_check_launch(ctx, "mg2d_lowrank_pack_a"); }
+    if (dtype == MG2D_C128) { MG2D_LR_CASES(CALL_D) }
+    else if (dtype == MG2D_C64) { MG2D_LR_CASES(CALL_F) }
+    else return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_lowrank_pack_a: bad dtype");
+#undef CALL_D
+#undef CALL_F
+    return mg2d_fail(ctx, MG2D_EUNSUPPORTED, "mg2d_lowrank_pack_a: (n, rank) must be (16,4) or (8,2)");
 }
 
 extern "C" int mg2d_relax_gs_strip(mg2d_ctx* ctx, void* phi, const void* phi_lo, const void* phi_hi, const void* D, const void* D0inv,

@@ -249,6 +249,19 @@ __global__ void twist_add_kernel(cplx<T>* __restrict__ D, T mu, long long S) {
     }
 }
 
+// a stored operator's twist set in place: Im D[s][0](i,i) = base[s][i] + delta Gamma5_c(i,i), Gamma5_c = diag(+1 x n/2, -1 x n/2),
+// summed in fp64 and rounded once to T (delta = 0 writes back the fp64 copy of the imaginary parts exactly)
+template <typename T>
+__global__ void twist_set_kernel(cplx<T>* __restrict__ D, const double* __restrict__ base, double delta, int n, long long S) {
+    const long long nel = S * n;
+    for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < nel; e += (long long)gridDim.x * blockDim.x) {
+        const long long s = e / n;
+        const int i = (int)(e - s * n);
+        const double v = base[e] + (2 * i < n ? delta : -delta);
+        D[(size_t)s * 5 * n * n + (size_t)i * n + i].y = (T)v;
+    }
+}
+
 template <typename T>
 int launch_wilson(mg2d_ctx* ctx, void* out, const void* in, const void* in_lo, const void* in_hi, const void* U,
                   const void* U_lo, const void* F, const void* b, double mass, bool tm, double mu, int Lx, int Ly, int mode,
@@ -373,6 +386,21 @@ extern "C" int mg2d_twist_add(mg2d_ctx* ctx, void* D, double mu, long long nsite
     else if (dtype == MG2D_C64) twist_add_kernel<float><<<(int)grid, 256, 0, st>>>((float2*)D, (float)mu, nsites);
     else return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_twist_add: bad dtype");
     return mg2d_check_launch(ctx, "mg2d_twist_add");
+}
+
+extern "C" int mg2d_twist_set(mg2d_ctx* ctx, void* D, const double* base, double delta, int n, long long nsites, int dtype,
+                              void* stream) {
+    if (!ctx) return MG2D_EINVAL;
+    if (!D || !base || nsites < 1 || !std::isfinite(delta)) return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_twist_set: bad argument");
+    if (n != 2 && n != 4 && n != 8 && n != 16 && n != 32)
+        return mg2d_fail(ctx, MG2D_EUNSUPPORTED, "mg2d_twist_set: n_dof must be one of 2,4,8,16,32");
+    cudaStream_t st = (cudaStream_t)stream;
+    const long long nel = nsites * n;
+    long long grid = (nel + 255) / 256; if (grid > (long long)ctx->num_sms * 8) grid = (long long)ctx->num_sms * 8;
+    if (dtype == MG2D_C128) twist_set_kernel<double><<<(int)grid, 256, 0, st>>>((double2*)D, base, delta, n, nsites);
+    else if (dtype == MG2D_C64) twist_set_kernel<float><<<(int)grid, 256, 0, st>>>((float2*)D, base, delta, n, nsites);
+    else return mg2d_fail(ctx, MG2D_EINVAL, "mg2d_twist_set: bad dtype");
+    return mg2d_check_launch(ctx, "mg2d_twist_set");
 }
 
 extern "C" int mg2d_wilson_relax_rb(mg2d_ctx* ctx, void* phi, const void* phi_lo, const void* phi_hi, const void* U,

@@ -16,7 +16,11 @@ flavours = 1 (RHMC): S_f = phi^dag r_{-1/2}(M) phi with M = D^dag D and r_p(x) =
 spectral range [a, b] (rational.py).  The heat bath draws eta as above and sets phi = r_{+1/4}(M) eta, so S_f(start) = |eta|^2;
 the force is sum_k alpha_k (-2 Re[Y_k^dag dD/dtheta X_k]) with X_k = (M + beta_k)^-1 phi from one multi-shift CG (rhmc.py) and
 Y_k = D X_k, one mg2d_hmc_momentum call per pole; the accept step is S_f(end) = alpha0 |phi|^2 + Re <phi, sum_k alpha_k x_k>.
-The multi-shift solves use the level-0 links only, so the coarse hierarchy is never refreshed.
+The multi-shift solves use the level-0 links only, so with mg_poles = 0 the coarse hierarchy is never refreshed.  mg_poles = K
+moves the K smallest MD poles to multigrid (rhmc.normal_solve: two FGCR solves per pole on the hierarchy re-twisted to
+-+sqrt(beta_k)); the multi-shift CG then keeps only the other poles, with the smallest of them as its base system.  The coarse
+levels are then refreshed after accepted trajectories as for two flavours.  The heat bath and the accept step stay on the
+precise multi-shift path.
 """
 from __future__ import annotations
 
@@ -30,7 +34,7 @@ from ._lib import MG2DError
 from .mg import MG, _ptr, _stream
 from .params import MGParams
 from .rational import MD_TOL, PRECISE_TOL, rational_approx
-from .rhmc import multishift_cg
+from .rhmc import multishift_cg, normal_solve
 
 _INV_ITER_STREAM = 2 ** 63 - 1       # counter stream of the start vector of the lambda_min estimate (trajectories use 3k + j)
 
@@ -44,12 +48,14 @@ class HMC:
     the force solves; accept_tol: of the final action's solve (and of the flavours = 1 heat bath).  spectrum = (a, b): the
     range of D^dag D the rational approximations of flavours = 1 cover (default: b = (|2+m| + 2 sqrt 2)^2, a rigorous bound, and
     a = 1/4 of lambda_min estimated at construction by inverse iteration with multigrid solves).  refresh_null_iters: sweeps of MG.refresh after an accepted trajectory (None: never refresh;
-    default 8, measured in DESIGN section 4).
+    default 8, measured in DESIGN section 4).  mg_poles (flavours = 1 only): the number K of smallest MD poles solved by
+    multigrid (normal_solve at md_tol) instead of the multi-shift CG; 0 (default) to the number of MD poles.
     precond_dtype / use_graph: passed to solve() (outer FGCR(8))."""
 
     def __init__(self, params: MGParams, theta, beta: float, tau: float = 1.0, n_md: int = 10, flavours: int = 2, seed: int = 1,
                  md_tol: float = 1e-10, accept_tol: float = 1e-12, refresh_null_iters: int | None = 8,
-                 precond_dtype: str | None = None, use_graph: bool = True, device: int | None = None, spectrum=None):
+                 precond_dtype: str | None = None, use_graph: bool = True, device: int | None = None, spectrum=None,
+                 mg_poles: int = 0):
         from . import setup
         p = params
         if p.stencil != "wilson":
@@ -74,6 +80,11 @@ class HMC:
             raise ValueError("need n_md >= 1 and tau > 0")
         if refresh_null_iters is not None and refresh_null_iters < 0:
             raise ValueError("refresh_null_iters must be None or >= 0")
+        if int(mg_poles) != mg_poles or mg_poles < 0:
+            raise ValueError(f"mg_poles must be an integer >= 0, got {mg_poles}")
+        if mg_poles and flavours != 1:
+            raise ValueError("mg_poles needs flavours=1 (one-flavour RHMC)")
+        self.mg_poles = int(mg_poles)
         self.p, self.L = p, p.L
         self.beta, self.tau, self.n_md, self.flavours, self.seed = float(beta), float(tau), int(n_md), int(flavours), int(seed)
         self.md_tol, self.accept_tol, self.refresh_null_iters = md_tol, accept_tol, refresh_null_iters
@@ -90,6 +101,8 @@ class HMC:
             c.close()
             self.mg = setup(U, p, init="device", device=dev)
         self.ctx = self.mg.ctx
+        if self.mg_poles:
+            self.mg._twist_state()           # kept from the links the coarse levels are built on (before update_links)
         self.mg.update_links(U)              # the hierarchy now owns its link tensor: the MD writes into it in place
         self.P = torch.empty((S, 2), dtype=torch.float64, device=self.device)
         self.theta0 = torch.empty_like(self.theta)
@@ -100,6 +113,7 @@ class HMC:
         self.u = torch.zeros(1, dtype=torch.complex128, device=self.device)
         self.k = 0                           # trajectories run
         self.stale = False                   # the links moved since the coarse hierarchy was last built for them
+        self._iters_mg = []                  # (-mu, +mu) FGCR iterations per MG pole of each force evaluation (mg_poles > 0)
         if self.flavours == 1:
             self._setup_rational(spectrum)
 
@@ -136,6 +150,8 @@ class HMC:
         self.r_md = rational_approx(-0.5, a, b, MD_TOL)
         self.r_acc = rational_approx(-0.5, a, b, PRECISE_TOL)
         self.r_hb = rational_approx(0.25, a, b, PRECISE_TOL)
+        if self.mg_poles > self.r_md.n:
+            raise ValueError(f"mg_poles = {self.mg_poles} exceeds the {self.r_md.n} poles of the MD approximation")
         self.phi = torch.empty_like(self.eta)
         self.red1 = torch.zeros(2, dtype=torch.float64, device=self.device)
 
@@ -154,10 +170,27 @@ class HMC:
         return info["iters"]
 
     def _force_one(self, eps, iters, timer):
-        mg, S, r = self.mg, self.L * self.L, self.r_md
-        with timer("solves"):
-            X, info = self._msc(self.phi, r, self.md_tol, False)
-        iters.append(info["iters"])
+        mg, S, r, K = self.mg, self.L * self.L, self.r_md, self.mg_poles
+        if K == 0:
+            with timer("solves"):
+                X, info = self._msc(self.phi, r, self.md_tol, False)
+            iters.append(info["iters"])
+        else:
+            Xs = []
+            if K < r.n:
+                with timer("solves"):
+                    Xm, info = multishift_cg(mg, self.phi, r.beta[K:], self.md_tol, self.MSC_MAX_ITERS)
+                if not info["converged"]:
+                    raise MG2DError(f"HMC: multi-shift solve did not converge in {info['iters']} iterations")
+                Xs = list(Xm)
+            iters.append(info["iters"] if K < r.n else 0)
+            with timer("mg_solves"):
+                Xg, ginfo = normal_solve(mg, self.phi, r.beta[:K], self.md_tol, precond_dtype=self.precond_dtype,
+                                         use_graph=self.use_graph)
+            timer.add("twist", ginfo["twist_ms"])
+            timer.add("mg_solves", -ginfo["twist_ms"])
+            self._iters_mg.append(ginfo["iters"])
+            X = list(Xg) + Xs
         with timer("momentum"):
             U = _ptr(mg.LVL[0].U)
             for k in range(r.n):
@@ -170,6 +203,13 @@ class HMC:
         mg, ctx, S, k = self.mg, self.ctx, self.L * self.L, self.k
         tm = _Timer(self.flavours)
         t_start = time.perf_counter()
+        refreshed = False
+        if self.mg_poles and self.stale and self.refresh_null_iters is not None:
+            with tm("refresh"):
+                mg.refresh(self.refresh_null_iters)
+            refreshed = True
+            self.stale = False
+        self._iters_mg = []
         red = self.red
         red.zero_()
         with tm("energies"):
@@ -203,6 +243,7 @@ class HMC:
         dH = H1 - H0
         accepted = bool(math.isfinite(dH) and u < math.exp(min(0.0, -dH)))
         if accepted:
+            self.stale = True
             plaq = r[5] / S
         else:
             self.theta.copy_(self.theta0)
@@ -216,7 +257,9 @@ class HMC:
         return {"trajectory": k, "dH": dH, "accepted": accepted, "exp_minus_dH": math.exp(-dH) if dH > -700 else float("inf"),
                 "plaquette": plaq, "H0": H0, "H1": H1, "iters_md": iters_md, "iters_accept": info["iters"],
                 "iters_heatbath": it_hb, "poles": (self.r_md.n, self.r_acc.n), "spectrum": self.spectrum, "ritz": info["ritz"],
-                "refreshed": False, "times_ms": dict(tm.totals(), total=1e3 * (time.perf_counter() - t_start))}
+                "iters_md_mg": self._iters_mg, "mg_poles": self.mg_poles, "refreshed": refreshed,
+                "times_ms": dict({"mg_solves": 0.0, "twist": 0.0, "refresh": 0.0}, **tm.totals(),
+                                 total=1e3 * (time.perf_counter() - t_start))}
 
     # ---- pieces --------------------------------------------------------------------------------------------
     def _solve(self, rhs, tol):
@@ -359,13 +402,21 @@ class _NullTimer:
     def __exit__(self, *exc):
         return False
 
+    @staticmethod
+    def add(name, ms):
+        pass
+
 
 class _Timer:
     """Device time of the phases of a trajectory (CUDA events, resolved once at the end).  The two solves of a force step are
     counted under 'solves'; the rest of that step is the momentum kernel."""
 
     def __init__(self, flavours):
-        self.ev, self.flavours = [], flavours
+        self.ev, self.flavours, self.extra = [], flavours, {}
+
+    def add(self, name, ms):
+        """Add a time measured elsewhere (ms) to `name`."""
+        self.extra[name] = self.extra.get(name, 0.0) + ms
 
     def __call__(self, name):
         t = self
@@ -385,7 +436,7 @@ class _Timer:
 
     def totals(self):
         torch.cuda.synchronize()
-        out = {}
+        out = dict(self.extra)
         for name, e0, e1 in self.ev:
             out[name] = out.get(name, 0.0) + e0.elapsed_time(e1)
         return out

@@ -25,7 +25,7 @@ import torch
 
 from . import _lib
 from ._lib import Context, MG2DError
-from .params import MGParams
+from .params import MGParams, replace_params
 from .rng import StdMT19937
 
 GCR_PAD = int(os.environ.get("MG2D_GCR_PAD", "0"))     # extra elements between stored FGCR directions (A/B knob; measured: no effect)
@@ -325,6 +325,22 @@ class Level:
         if self.F is not None:
             self._ensure_D0inv()       # (a precision copy receives F but builds its own D0^-1 for the c = D0^-1 r pass)
         return self.F is not None
+
+    def retwist(self, base: torch.Tensor, delta: float, A: torch.Tensor | None):
+        """Self blocks of the stored operator set to base + delta Gamma5_c on the imaginary diagonal (mg2d_twist_set), then
+        every buffer derived from them rebuilt in place: D0^-1, M, the -D0^-1 A half of F (from the kept factors A) and the
+        half-precision copies."""
+        mg, call, st = self.mg, self.mg.ctx.call, _stream()
+        call("mg2d_twist_set", _ptr(self.D), _ptr(base), float(delta), self.n, self.S, mg.dcode, st)
+        if self.D0inv is not None:
+            call("mg2d_block_inverse", _ptr(self.D0inv), _ptr(self.D), self.n, self.S, mg.dcode, st)
+        if self.M is not None:
+            call("mg2d_premultiply", _ptr(self.M), _ptr(self.D), _ptr(self.D0inv), self.n, self.S, mg.dcode, st)
+        if self.F is not None and A is not None:
+            call("mg2d_lowrank_pack_a", _ptr(self.F), _ptr(A), _ptr(self.D0inv), self.n, self.lr_rank, self.S, mg.dcode, st)
+        if self.Dh is not None:
+            call("mg2d_to_half", _ptr(self.Dh), _ptr(self.D), self.D.numel(), st)
+            call("mg2d_to_half", _ptr(self.D0inv_h), _ptr(self.D0inv), self.D0inv.numel(), st)
 
     def hop_factors(self, lvl_f: "Level", P: torch.Tensor, p_lo: int, p_hi: int):
         """Rank-`block` factors of this level's hopping blocks from the fine operator and projector (mg2d_hop_factors);
@@ -780,6 +796,7 @@ class MG:
             self._drop_graphs()
             self.info["own_links"] = True
         lv0.U.copy_(U)
+        self.info["links_moved"] = True
         sh = self.info.get("single")
         if isinstance(sh, MG):
             sh.LVL[0].U.copy_(lv0.U)
@@ -798,6 +815,8 @@ class MG:
         self._drop_graphs()
         for lv in self.LVL:
             lv.Dh = lv.D0inv_h = None
+        self.info.pop("links_moved", None)
+        retwisted = self.info.pop("twist", None) is not None
         if self.p.nlevels == 0:
             return
         lv0 = self.LVL[0]
@@ -806,16 +825,84 @@ class MG:
             compute_near_null(self, self.p.quad, gen_null=0)
         else:
             compute_near_null(self, self.p.quad, gen_null=1, null_iters=null_iters, warm=True)
+        if retwisted:          # the hierarchy is now built at the current twist: keep set_twist working from there
+            self._twist_state()
+
+    # ---- changing the twisted mass of a built hierarchy --------------------------------------------------
+    def _twist_state(self) -> dict:
+        """What set_twist keeps, taken once: the build twist mu_b, the fp64 imaginary self-block diagonals of every stored
+        operator and the factors A of the first coarse level's low-rank hopping blocks (setup discards them; they are rebuilt
+        here from a transient stored level-0 operator with mg2d_hop_factors).  A must come from the links the coarse levels were
+        built on, so the state cannot be taken once update_links moved them (refresh rebuilds the levels and re-takes it)."""
+        st = self.info.get("twist")
+        if st is not None:
+            return st
+        p = self.p
+        if self.comm is not None:
+            raise MG2DError("set_twist: strip-decomposed hierarchies (DistMG) are not supported")
+        if p.ntl:
+            raise MG2DError("set_twist: non-telescoping hierarchies are not supported")
+        if p.stencil != "wilson":
+            raise MG2DError("set_twist: the twisted mass exists for the Wilson stencil only")
+        if self.info.get("links_moved"):
+            raise MG2DError("set_twist: the links moved since the coarse levels were built; call refresh() first")
+        base = [None if lv.D is None else lv.D[:, 0].diagonal(dim1=-2, dim2=-1).imag.to(torch.float64).contiguous()
+                for lv in self.LVL]
+        A = [None] * len(self.LVL)
+        for lv in self.LVL[1:]:
+            if lv.F is None or not lv.lr_rank:
+                continue
+            lf = self.LVL[lv.lvl - 1]
+            Df = lf.D
+            if Df is None:     # matrix-free level 0: the hopping blocks of the stored operator (mass, clover and twist unused)
+                Df = torch.empty((lf.S, 5, lf.n, lf.n), dtype=self.tdtype, device=self.device)
+                self.ctx.call("mg2d_lvl0_matrix", _ptr(Df), _ptr(lf.U), lf.U_lo_ptr, float(p.mass), 0, lf.L, lf.Ly, self.dcode,
+                              _stream())
+            P = lf.phi_null
+            p_lo, p_hi = lf._halo(P, 1, lf.nc * lf.n)
+            A[lv.lvl] = torch.empty((lv.S, 4 * lf.block, lv.n), dtype=self.tdtype, device=self.device)
+            B = torch.empty_like(A[lv.lvl])
+            self.ctx.call("mg2d_hop_factors", _ptr(A[lv.lvl]), _ptr(B), _ptr(Df), _ptr(P), p_lo, p_hi, lf.n, lv.n, lf.L, lf.Ly,
+                          lf.block, self.dcode, _ptr(self.status[1:]), _stream())
+            del B, Df
+        st = self.info["twist"] = {"mu_b": p.mu, "base": base, "A": A}
+        return st
+
+    def set_twist(self, mu: float):
+        """Change the twisted mass of the built hierarchy to mu in place: D_tm(mu) = D + i mu gamma5 on level 0 (the matrix-free
+        tm entry points read p.mu), i mu Gamma5_c on the coarse self blocks (exact on the chirality-split projectors), with D0^-1,
+        M, F and the half-precision copies rebuilt in their buffers, here and on the complex64 shadow.  No Galerkin product is
+        recomputed.  The first call keeps the state of _twist_state (on the benchmark's 4096^2 hierarchy mostly the 4.3 GB of A).
+        Captured graphs are kept per twist: returning to a twist replays the graphs captured there."""
+        mu = float(mu)
+        if not math.isfinite(mu):
+            raise ValueError(f"set_twist: mu must be finite (mu {mu})")
+        st = self._twist_state()
+        if mu == self.p.mu:
+            return
+        delta = mu - st["mu_b"]
+        for lv in self.LVL:
+            if lv.D is not None:
+                lv.retwist(st["base"][lv.lvl], delta, st["A"][lv.lvl])
+        self.p = replace_params(self.p, mu=mu)
+        sh = self.info.get("single")
+        if isinstance(sh, MG):
+            # the same fp64 sum rounded to complex64 equals the cast of the complex128 result; F is cast as make_single_precision does
+            for lv, l32 in zip(self.LVL, sh.LVL):
+                if l32.D is not None:
+                    l32.retwist(st["base"][lv.lvl], delta, None)
+                if l32.F is not None:
+                    sh.ctx.call("mg2d_convert", _ptr(l32.F), _lib.C64, _ptr(lv.F), _lib.C128, lv.F.numel(), _stream())
+            sh.p = replace_params(sh.p, mu=mu)
 
 
 def make_single_precision(mg: "MG") -> "MG":
     """complex64 shadow of a set-up hierarchy (links, clover field, stored operators, projectors), used as the preconditioner
     of the fp64 outer GCR: every V-cycle kernel then moves half the bytes.  The outer residual, the GCR vectors
     and the convergence test stay in complex128, so the 1e-10 TRUE residual is unaffected."""
-    import dataclasses
     if mg.p.dtype != "complex128":
         raise ValueError("make_single_precision expects a complex128 hierarchy")
-    p32 = dataclasses.replace(mg.p, dtype="complex64", size=[], n_dof=[])
+    p32 = replace_params(mg.p, dtype="complex64")
     if mg.comm is not None:
         from .dist import DistMG
         m32 = DistMG(p32, mg.comm, min_rows=mg.min_rows, plan=mg.plan)
@@ -1199,9 +1286,9 @@ def _perform_MG(mg: MG, tol: float | None = None, max_iters: int | None = None, 
     ntl = p.ntl and p.nlevels > 0
     cyc = None
     if use_graph:
-        cyc = mg.info.get("cycle_graph")
+        cyc = mg.info.get(("cycle_graph", p.mu))          # a graph bakes the level-0 twist into its launches
         if cyc is None:
-            cyc = mg.info["cycle_graph"] = CycleGraph(mg)
+            cyc = mg.info[("cycle_graph", p.mu)] = CycleGraph(mg)
     it = 0
     while it < max_iters:
         nb = min(check_every, max_iters - it)
@@ -1353,7 +1440,8 @@ def gcr_MG(mg: MG, tol: float | None = None, max_iters: int | None = None, resta
 
     graphs = None
     if use_graph and pm.p.smoother != "gs":
-        gkey = ("iter_graphs", id(pm), lazy, pm.use_half, pm.lowrank, pm.premul, pm.persistent_sites, restart, tuple(pm.p.pre), tuple(pm.p.post))
+        gkey = ("iter_graphs", id(pm), lazy, pm.use_half, pm.lowrank, pm.premul, pm.persistent_sites, restart, tuple(pm.p.pre), tuple(pm.p.post),
+                p.mu)
         graphs = mg.info.setdefault(gkey, {})
     info = {"iters": 0, "resnorms": [], "ntl_weights": [], "converged": False, "diverged": False}
     bn2 = None

@@ -7,6 +7,7 @@ meanings; `from_argv` accepts the reference's argv order.
 """
 from __future__ import annotations
 
+import dataclasses
 import math
 from dataclasses import dataclass, field
 
@@ -115,6 +116,12 @@ class MGParams:
     def diag(self) -> float:
         """D0 of level 0: 1/scale[0] (S6/params.h:76,82), with the sign of S6/level.h:148,165."""
         return (2.0 + self.mass) if self.stencil == "wilson" else -(4.0 + self.mass)
+
+
+def replace_params(p: MGParams, **changes) -> MGParams:
+    """dataclasses.replace that keeps a per-level block list: __post_init__ leaves only its first entry in p.block, so replace()
+    alone would rebuild the level sizes from one block size."""
+    return dataclasses.replace(p, block=list(p.blocks) if p.nlevels > 0 else p.block, **changes)
 
 
 def make_params(L, mass, stencil="wilson", nlevels=2, block=2, n_null=None, n_smooth=3, smoother="gs", ntl=False,

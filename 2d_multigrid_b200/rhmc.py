@@ -4,6 +4,11 @@ Jegerlehner's multi-shift CG (hep-lat/9612014): one Krylov space for every shift
 iteration is two existing Wilson applies and mg2d_gamma5 for M p_0 = gamma5 D gamma5 D p_0 (D^dag = gamma5 D gamma5), then the
 two vector passes of csrc/rhmc.cu; the scalar recurrences run on the device and the host reads one residual norm per
 iteration.  Every x_k starts from 0.  The coarse levels of the hierarchy are never touched.
+
+normal_solve solves the same systems with the multigrid hierarchy instead: D_tm(mu)^dag D_tm(mu) = D^dag D + mu^2 and
+D_tm(mu)^dag = gamma5 D_tm(-mu) gamma5 give, for sigma = mu^2,
+    (D^dag D + sigma)^-1 = D_tm(+mu)^-1 gamma5 D_tm(-mu)^-1 gamma5,
+two FGCR solves on one hierarchy whose twist MG.set_twist changes in place.
 """
 from __future__ import annotations
 
@@ -98,9 +103,20 @@ def multishift_cg(mg, rhs, shifts, tol: float, max_iters: int, weights=None):
     info["residuals"] = [res_sorted[inv[k]] for k in range(N)]
     if acc:
         return y, info
-    # true residuals, once: rhs - (M + s_k) x_k
-    out = torch.zeros(N, dtype=torch.float64, device=dev)
-    for j in range(N):
+    tr = _true_residuals(mg, phi, X, sig, b2, (t, u, w))
+    info["true_residuals"] = [tr[inv[k]] for k in range(N)]
+    if order != list(range(N)):
+        X = X[torch.tensor(inv, device=dev)]
+    return X, info
+
+
+def _true_residuals(mg, phi, X, sig, b2, work):
+    """|phi - (D^dag D + sig[j]) X[j]| / |phi| for every j, computed once (b2 = |phi|^2; work: three fields)."""
+    lv, ctx, st = mg.LVL[0], mg.ctx, _stream()
+    S = lv.S
+    t, u, w = work
+    out = torch.zeros(len(sig), dtype=torch.float64, device=phi.device)
+    for j in range(len(sig)):
         lv._stencil(t, X[j], None, _lib.MODE_APPLY, None)
         ctx.call("mg2d_gamma5", _ptr(u), _ptr(t), S, st)
         lv._stencil(w, u, None, _lib.MODE_APPLY, None)
@@ -109,10 +125,101 @@ def multishift_cg(mg, rhs, shifts, tol: float, max_iters: int, weights=None):
         ctx.call("mg2d_axpy", _ptr(t), _ptr(w), -1.0, 0.0, None, 2 * S, _lib.C128, st)
         ctx.call("mg2d_axpy", _ptr(t), _ptr(X[j]), -sig[j], 0.0, None, 2 * S, _lib.C128, st)
         ctx.call("mg2d_norm2", _ptr(t), 2 * S, _lib.C128, _ptr(out[j:]), st)
-    tr = [math.sqrt(v / b2) for v in out.tolist()]
-    info["true_residuals"] = [tr[inv[k]] for k in range(N)]
-    if order != list(range(N)):
-        X = X[torch.tensor(inv, device=dev)]
+    return [math.sqrt(v / b2) for v in out.tolist()]
+
+
+def operator_norm_bound(p, mu: float) -> float:
+    """An upper bound on the operator norm of D_tm(mu) = D + i mu gamma5: |2+m| + |c_sw|/2 for the self term (the clover field is
+    at most |c_sw|/2), 2 sqrt 2 for the four hops and |mu|."""
+    return abs(2.0 + p.mass) + abs(p.csw) / 2.0 + 2.0 * math.sqrt(2.0) + abs(mu)
+
+
+def second_solve_tol(tol: float, rhs_norm: float, z_norm: float, p, mu: float) -> float:
+    """Relative tolerance of the second solve D_tm(+mu) x = gamma5 z.  With r1 = gamma5 rhs - D_tm(-mu) z and
+    r2 = gamma5 z - D_tm(+mu) x the normal residual is rhs - (D^dag D + mu^2) x = gamma5 r1 + D_tm(mu)^dag r2, so |r1| <= tol/2 |rhs|
+    and |r2| <= this value times |z| bound it by tol |rhs|."""
+    return tol * rhs_norm / (2.0 * operator_norm_bound(p, mu) * z_norm)
+
+
+_SOLVE_KW = ("precond_dtype", "use_graph", "max_iters", "restart", "check_every")
+
+
+def normal_solve(mg, rhs, shifts, tol: float, **solve_kw):
+    """Solve (D^dag D + shifts[k]) x_k = rhs for every k with multigrid: x = D_tm(+mu)^-1 gamma5 D_tm(-mu)^-1 gamma5 rhs with
+    mu = sqrt(shifts[k]), each a solve(outer="gcr") from x0 = 0 with solve_kw (precond_dtype, use_graph, max_iters, restart,
+    check_every) on the hierarchy `mg`, whose twist set_twist changes in place.  The first solve runs to tol/2, the second to
+    second_solve_tol, so that the true residual of the normal equations is at most tol.
+
+    mg: a one-GPU Wilson or Wilson-clover hierarchy at twist 0 (p.mu == 0), left at twist 0.  rhs[L*L, 2] complex128;
+    shifts: numbers >= 0 (0 is the two-flavour composition D^-1 gamma5 D^-1 gamma5).  Returns (X[N, L*L, 2] in the order of
+    shifts, info) with info: iters (the (-mu, +mu) FGCR iterations per shift), converged, true_residuals (relative
+    |rhs - (D^dag D + s_k) x_k| / |rhs|, computed once at the end) and twist_ms (device time spent in set_twist).
+    Raises MG2DError when an inner solve does not converge."""
+    from . import solve
+    p = mg.p
+    if p.stencil != "wilson" or p.dtype != "complex128":
+        raise ValueError("normal_solve needs a complex128 Wilson hierarchy")
+    if p.mu != 0.0:
+        raise ValueError(f"normal_solve needs the hierarchy at twist 0 (D itself); it is at mu = {p.mu}")
+    if mg.comm is not None:
+        raise ValueError("normal_solve runs on one GPU (whole lattice)")
+    lv = mg.LVL[0]
+    shifts = [float(s) for s in shifts]
+    if not shifts or not all(s >= 0.0 and math.isfinite(s) for s in shifts):
+        raise ValueError("need at least one finite shift >= 0")
+    if not tol > 0.0:
+        raise ValueError("need tol > 0")
+    bad = sorted(set(solve_kw) - set(_SOLVE_KW))
+    if bad:
+        raise ValueError(f"normal_solve: unknown solve arguments {bad} (allowed: {', '.join(_SOLVE_KW)})")
+    ctx, S, st = mg.ctx, lv.S, _stream()
+    dev = mg.device
+    phi = torch.as_tensor(rhs).to(torch.complex128).to(dev).reshape(S, 2)
+    nrm = torch.zeros(2, dtype=torch.float64, device=dev)
+    ctx.call("mg2d_norm2", _ptr(phi), 2 * S, _lib.C128, _ptr(nrm), st)
+    b2 = float(nrm[0].item())
+    if not b2 > 0.0:
+        raise ValueError("normal_solve: rhs is zero")
+    X = torch.empty((len(shifts), S, 2), dtype=torch.complex128, device=dev)
+    g = torch.empty_like(phi)
+    ctx.call("mg2d_gamma5", _ptr(g), _ptr(phi), S, st)
+    events = []
+
+    def twist(mu):
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        mg.set_twist(mu)
+        e1.record()
+        events.append((e0, e1))
+
+    def inner(b, t, what):
+        x, info = solve(mg, rhs=b, tol=t, outer="gcr", **solve_kw)
+        if not info["converged"]:
+            raise MG2DError(f"normal_solve: the {what} solve did not converge (iterations {info['iters']}, residual "
+                            f"{info['resnorms'][-1] if info['resnorms'] else float('nan'):.3g})")
+        return x, info["iters"]
+    iters = []
+    gz = torch.empty_like(phi)
+    try:
+        for k, s in enumerate(shifts):
+            mu = math.sqrt(s)
+            twist(-mu)
+            z, n1 = inner(g, 0.5 * tol, "D_tm(-mu)")
+            ctx.call("mg2d_norm2", _ptr(z), 2 * S, _lib.C128, _ptr(nrm[1:]), st)
+            ctx.call("mg2d_gamma5", _ptr(gz), _ptr(z), S, st)
+            z2 = float(nrm[1].item())
+            twist(mu)
+            t2 = second_solve_tol(tol, math.sqrt(b2), math.sqrt(z2), p, mu) if z2 > 0.0 else 1.0
+            x, n2 = inner(gz, t2, "D_tm(+mu)")
+            ctx.call("mg2d_copy", _ptr(X[k]), _ptr(x), 2 * S, _lib.C128, st)
+            iters.append((n1, n2))
+    finally:
+        twist(0.0)
+    work = (g, gz, torch.empty_like(phi))
+    tr = _true_residuals(mg, phi, X, shifts, b2, work)
+    torch.cuda.synchronize()
+    info = {"iters": iters, "converged": True, "true_residuals": tr,
+            "twist_ms": sum(e0.elapsed_time(e1) for e0, e1 in events)}
     return X, info
 
 

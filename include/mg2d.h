@@ -101,6 +101,11 @@ int mg2d_wilson_tm_relax_rb2(mg2d_ctx*, void* out, const void* in, const void* i
                              const void* F_hi, const void* r, const void* r_lo, const void* r_hi, double mass, double mu,
                              int Lx, int Ly, int yoff, int dtype, const struct mg2d_halo_link* link, void* stream);
 int mg2d_twist_add(mg2d_ctx*, void* D, double mu, long long nsites, int dtype, void* stream);
+/* Twist of a built hierarchy changed in place (MG.set_twist): Im D[s][0](i,i) = base[s][i] + delta Gamma5_c(i,i) for a stored
+ * operator with n in {2,4,8,16,32} (column-major blocks), Gamma5_c = diag(+1 x n/2, -1 x n/2) (n = 2: sigma3 of level 0).
+ * base [nsites][n] fp64 holds the imaginary diagonal at the build twist mu_b and delta = mu - mu_b (finite); the sum is formed
+ * in fp64 and rounded once to dtype, so delta = 0 restores the operator bit for bit.  Real parts are not touched. */
+int mg2d_twist_set(mg2d_ctx*, void* D, const double* base, double delta, int n, long long nsites, int dtype, void* stream);
 
 /* ---- generic 5-point block stencil (all coarse levels; level 0 in reference-compat mode) -------------- */
 /* Level::f_apply_D / f_residue, n in {1,2,4,8,16,32}; nvec vectors `vstride` elements apart. */
@@ -180,6 +185,10 @@ int mg2d_hop_factors(mg2d_ctx*, void* A, void* B, const void* Df, const void* P,
                      int nf, int nc, int Lxf, int Lyf, int block, int dtype, int* status, void* stream);
 int mg2d_lowrank_pack(mg2d_ctx*, void* F, const void* A, const void* B, const void* D0inv, int n, int rank,
                       long long nsites, int dtype, void* stream);
+/* mg2d_lowrank_pack_a: only the -D0inv A half of F (after D0inv changed; the conj(B) half does not depend on the self
+ * blocks), bit-identical to what mg2d_lowrank_pack writes there. */
+int mg2d_lowrank_pack_a(mg2d_ctx*, void* F, const void* A, const void* D0inv, int n, int rank, long long nsites, int dtype,
+                        void* stream);
 int mg2d_relax_rb_lr(mg2d_ctx*, void* phi, const void* phi_lo, const void* phi_hi, const void* F, const void* D0inv,
                      const void* r, void* cbuf, int cmode, int n, int rank, int Lx, int Ly, int colour, int yoff,
                      int dtype, int nvec, long long vstride, long long hstride, const struct mg2d_halo_link* link, void* stream);

@@ -18,7 +18,7 @@ nl = p.nlevels
 def run(pre, post, mixed, restart=8):
     for m in [mg] + ([mg.info["single"]] if "single" in mg.info else []):
         m.p.pre, m.p.post = list(pre), list(post)
-        m.info.pop("precond_graph", None); m.info.pop("cycle_graph", None)
+        m.info.pop("precond_graph", None); m.info.pop(("cycle_graph", m.p.mu), None)
     kw = dict(rhs=rhs, tol=1e-10, outer="gcr", restart=restart, use_graph=True, check_every=1, max_iters=120)
     if mixed: kw["precond_dtype"] = "complex64"
     x, info = mg2d.solve(mg, **kw)
