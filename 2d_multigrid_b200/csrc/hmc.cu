@@ -76,7 +76,8 @@ hmc_links_kernel(double* __restrict__ theta, const double* __restrict__ P, doubl
     }
 }
 
-__global__ void gamma5_kernel(C* __restrict__ out, const C* __restrict__ in, long long S) {
+// out may equal in (mg2d.h): no __restrict__, so `in` is not read through the non-coherent load path
+__global__ void gamma5_kernel(C* out, const C* in, long long S) {
     for (long long s = blockIdx.x * (long long)blockDim.x + threadIdx.x; s < S; s += (long long)gridDim.x * blockDim.x) {
         const C v1 = in[2 * s + 1];
         out[2 * s] = in[2 * s];
