@@ -49,6 +49,16 @@ struct Rb2Args {
     T tz_re, tz_im;                              // TM: 1/(2+m + i mu) (two reals: a complex member would realign the struct)
 };
 
+// a * b and conj(a) * b with the rounding written out: each component is fma(first product, second product rounded).  Left
+// to the compiler, which of the two products is fused follows the instruction schedule, and it differed between the LINKED
+// and the unlinked instantiation: a strip relaxed to last-bit different values than the same rows on one GPU.
+template <typename C> __device__ __forceinline__ C rb2_mul(C a, C b) {
+    C r; r.x = fma(a.x, b.x, -(a.y * b.y)); r.y = fma(a.x, b.y, a.y * b.x); return r;
+}
+template <typename C> __device__ __forceinline__ C rb2_mulc(C a, C b) {
+    C r; r.x = fma(a.x, b.x, a.y * b.y); r.y = fma(a.x, b.y, -(a.y * b.x)); return r;
+}
+
 template <typename T>
 __device__ __forceinline__ const cplx<T>* rb2_row(const cplx<T>* f, const cplx<T>* lo2, const cplx<T>* hi, int y, int Lx, int Ly) {
     if (y < 0) return lo2 + (size_t)(y + 2) * Lx * 2;
@@ -81,10 +91,10 @@ __device__ __forceinline__ Spinor<T> rb2_update(cplx<T> ux, cplx<T> a_xp, cplx<T
                                                 T inv_diag, const Rb2Args<T>& a, int y) {
     using C = cplx<T>;
     const T half = (T)0.5;
-    const C A = cmul(ux, a_xp);
+    const C A = rb2_mul(ux, a_xp);
     const C B = wb_xm;
-    const C Cc = cmul(uy, cadd(qyp.c0, cmul_i(qyp.c1)));
-    const C Dd = cmulc(uym, csub(qym.c0, cmul_i(qym.c1)));
+    const C Cc = rb2_mul(uy, cadd(qyp.c0, cmul_i(qyp.c1)));
+    const C Dd = rb2_mulc(uym, csub(qym.c0, cmul_i(qym.c1)));
     const C h0 = cadd(cadd(A, B), cadd(Cc, Dd));
     const C h1 = cadd(csub(B, A), cmul_i(csub(Dd, Cc)));
     T i0 = inv_diag, i1 = inv_diag;
@@ -98,7 +108,7 @@ __device__ __forceinline__ Spinor<T> rb2_update(cplx<T> ux, cplx<T> a_xp, cplx<T
         tm_self_inverse<T>(SW ? rb2_f<T>(a, y, x) : (T)0, a.diag, a.mu, mk<T>(a.tz_re, a.tz_im), z0, z1);
         C t0 = mk<T>(-half * h0.x, -half * h0.y), t1 = mk<T>(-half * h1.x, -half * h1.y);
         if (HAS_R) { const Spinor<T> rr = load_spinor<T>(r_row, (size_t)x); t0 = cadd(rr.c0, t0); t1 = cadd(rr.c1, t1); }
-        o.c0 = cmul(t0, z0); o.c1 = cmul(t1, z1);
+        o.c0 = rb2_mul(t0, z0); o.c1 = rb2_mul(t1, z1);
     } else if (HAS_R) {
         const Spinor<T> rr = load_spinor<T>(r_row, (size_t)x);
         o.c0.x = (rr.c0.x - half * h0.x) * i0; o.c0.y = (rr.c0.y - half * h0.y) * i0;
@@ -211,29 +221,29 @@ wilson_rb2_kernel(Rb2Args<T> a) {
                 C a_here = csub(bk_0.c0, bk_0.c1);
                 C a_xp = shfl_c(a_here, lane + 1);
                 if (lane == 31) { const Spinor<T> q = rb2_phi<T>(a, rho, xp_out, linked); a_xp = csub(q.c0, q.c1); }
-                const C wb = cmulc(u0_ux0, cadd(bk_0.c0, bk_0.c1));
+                const C wb = rb2_mulc(u0_ux0, cadd(bk_0.c0, bk_0.c1));
                 rd_0 = rb2_update<T, HAS_R, SW, TM>(u0_ux1, a_xp, wb, u0_uy1, bk_p, um_uy1, bk_m, rrow, x1, a.inv_diag, a, rho);
                 if (do_black) {
                     // ---- stage B(rho-1): target c1 of row rho-1; red sources of that row sit in c0 (rd_m)
                     a_here = csub(rd_m.c0, rd_m.c1);
                     a_xp = shfl_c(a_here, lane + 1);
-                    const C wbm = cmulc(um_ux0, cadd(rd_m.c0, rd_m.c1));
+                    const C wbm = rb2_mulc(um_ux0, cadd(rd_m.c0, rd_m.c1));
                     const Spinor<T> nb = rb2_update<T, HAS_R, SW, TM>(um_ux1, a_xp, wbm, um_uy1, rd_0, umm_uy1, rd_mm, rrow_m, x1, a.inv_diag, a, rho - 1);
                     rb2_store<T>(a, rho - 1, x0, x1, act0, act1, rd_m, nb, push_lo, push_hi);
                 }
             } else {
                 // ---- stage R(rho): target c0; +x source = own c1 (bk_0), -x source = lane-1's c1
-                C wb_here = cmulc(u0_ux1, cadd(bk_0.c0, bk_0.c1));
+                C wb_here = rb2_mulc(u0_ux1, cadd(bk_0.c0, bk_0.c1));
                 C wb_xm = shfl_c(wb_here, lane - 1);
                 if (lane == 0) {
                     const Spinor<T> q = rb2_phi<T>(a, rho, xm_out, linked);
-                    wb_xm = cmulc(__ldg(urow + 2 * (size_t)xm_out), cadd(q.c0, q.c1));
+                    wb_xm = rb2_mulc(__ldg(urow + 2 * (size_t)xm_out), cadd(q.c0, q.c1));
                 }
                 const C ap = csub(bk_0.c0, bk_0.c1);
                 rd_0 = rb2_update<T, HAS_R, SW, TM>(u0_ux0, ap, wb_xm, u0_uy0, bk_p, um_uy0, bk_m, rrow, x0, a.inv_diag, a, rho);
                 if (do_black) {
                     // ---- stage B(rho-1): target c0 of row rho-1; red sources of that row sit in c1 (rd_m)
-                    wb_here = cmulc(um_ux1, cadd(rd_m.c0, rd_m.c1));
+                    wb_here = rb2_mulc(um_ux1, cadd(rd_m.c0, rd_m.c1));
                     wb_xm = shfl_c(wb_here, lane - 1);
                     const C apm = csub(rd_m.c0, rd_m.c1);
                     const Spinor<T> nb = rb2_update<T, HAS_R, SW, TM>(um_ux0, apm, wb_xm, um_uy0, rd_0, umm_uy0, rd_mm, rrow_m, x0, a.inv_diag, a, rho - 1);
